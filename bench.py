@@ -22,6 +22,11 @@ One "step" = one pass of the hot path over that batch.
   queue_e2e the gateway plugin path (GatewayCompressHash workers behind a GatewayQueue, chunk files on tmpfs), a bounded
             stream, run as a subprocess after the timed regions (rank 0 only).
 Only the cpu_baseline / --impl reference legs touch oracle/.
+
+--dump-outputs DIR  writes what the last timed step of `value` (and of config3, prefixed config3_) handed back, as .npy
+            (rank 0): frame_lens (float64, one per chunk), md5 (float32 bytes, chunks x 16) and frame_bytes_sample (float32,
+            chunks x up to 4096 bytes of each frame at fixed, seeded relative positions).  Inputs are seeded, so two builds
+            run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -37,6 +42,7 @@ from pathlib import Path
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True  # the benchmark leaves the tree as it found it (it may be read-only); forked workers inherit this
 
 METRIC = "chunk-pipeline GB/s (raw input)"
 UNIT = "GB/s"
@@ -306,9 +312,28 @@ def fill_device_input(torch, native, dev, workload, n_chunks, chunk_bytes, rank)
     return d_in, stride_in
 
 
-def device_resident_run(torch, native, dev, local, workload, n_chunks, chunk_bytes, rank, steps, warmup, sample_clocks=True, verify_decode=False):
+DUMP_SAMPLE_BYTES = 4 << 20  # frame bytes sampled per record: 16 MiB as float32, so value + config3 stay under 64 MB
+
+
+def sample_outputs(torch, np, d_out, dst_off, out_lens, digests) -> dict:
+    """What a caller of the device path holds after a step, as float arrays: every frame length and digest, and each frame's
+    bytes at the same fixed, seeded relative positions."""
+    n = len(out_lens)
+    m = max(1, min(4096, DUMP_SAMPLE_BYTES // n))
+    u = np.sort(np.random.default_rng(0).random(m))
+    lens = np.asarray(out_lens, dtype=np.int64)
+    pos = np.asarray(dst_off, dtype=np.int64)[:, None] + (u[None, :] * lens[:, None]).astype(np.int64)
+    sample = d_out[torch.from_numpy(pos.ravel()).to(d_out.device)].float().cpu().numpy().reshape(n, m)
+    md5 = np.frombuffer(b"".join(digests), dtype=np.uint8).reshape(n, 16).astype(np.float32)
+    return {"frame_lens": lens.astype(np.float64), "md5": md5, "frame_bytes_sample": sample}
+
+
+def device_resident_run(torch, native, dev, local, workload, n_chunks, chunk_bytes, rank, steps, warmup, sample_clocks=True, verify_decode=False,
+                        dump=False):
     """K timed passes of the fused kernel over a batch resident in HBM, CUDA events on the launching stream."""
     import hashlib
+
+    import numpy as np
 
     d_in, stride_in = fill_device_input(torch, native, dev, workload, n_chunks, chunk_bytes, rank)
     bound = native.frame_bound(chunk_bytes)
@@ -324,21 +349,7 @@ def device_resident_run(torch, native, dev, local, workload, n_chunks, chunk_byt
         return ctx.process_device(d_in.data_ptr(), src_off, lens, d_out.data_ptr(), dst_off, caps, 0, stream)
 
     for _ in range(warmup):
-        out_lens, digests, _ = step()
-    # parity spot check outside the timed region (hashlib is stdlib, not the oracle)
-    host0 = d_in[:chunk_bytes].cpu().numpy().tobytes()
-    if digests[0] != hashlib.md5(host0).digest():
-        raise SystemExit("MD5 mismatch against hashlib on chunk 0 -- refusing to report a number")
-    roundtrip = None
-    if verify_decode:
-        # the frames just produced, decoded by the receiver-side kernels, must give the input back (+ the same digests)
-        k = min(n_chunks, 64)
-        d_back = torch.empty(k * stride_in + 64, dtype=torch.uint8, device=dev)
-        st, dg2, _ = ctx.decode_device(d_out.data_ptr(), dst_off[:k], out_lens[:k], d_back.data_ptr(), src_off[:k], lens[:k], 0)
-        roundtrip = all(x == 0 for x in st) and dg2 == digests[:k] and bool(torch.equal(d_back[: k * stride_in - (stride_in - chunk_bytes)], d_in[: k * stride_in - (stride_in - chunk_bytes)]))
-        del d_back
-        if not roundtrip:
-            raise SystemExit("LZ4 frames do not decode back to the input -- refusing to report a number")
+        step()
     sampler = ClockSampler(local) if sample_clocks else None
     torch.cuda.synchronize()
     if sampler:
@@ -354,8 +365,24 @@ def device_resident_run(torch, native, dev, local, workload, n_chunks, chunk_byt
     torch.cuda.synchronize()
     elapsed = ev0.elapsed_time(ev1) / 1e3
     clocks = sampler.stop() if sampler else None
-    res = {"elapsed": elapsed, "kernel_ms": statistics.mean(kernel_ms), "frame_bytes": sum(out_lens), "launches": ctx.launches - launches0,
-           "clocks": clocks, "roundtrip": roundtrip, "total_in": n_chunks * chunk_bytes}
+    launches = ctx.launches - launches0
+    # parity spot check of the last timed step, outside the timed region (hashlib is stdlib, not the oracle)
+    host0 = d_in[:chunk_bytes].cpu().numpy().tobytes()
+    if digests[0] != hashlib.md5(host0).digest():
+        raise SystemExit("MD5 mismatch against hashlib on chunk 0 -- refusing to report a number")
+    roundtrip = None
+    if verify_decode:
+        # the frames just produced, decoded by the receiver-side kernels, must give the input back (+ the same digests)
+        k = min(n_chunks, 64)
+        d_back = torch.empty(k * stride_in + 64, dtype=torch.uint8, device=dev)
+        st, dg2, _ = ctx.decode_device(d_out.data_ptr(), dst_off[:k], out_lens[:k], d_back.data_ptr(), src_off[:k], lens[:k], 0)
+        roundtrip = all(x == 0 for x in st) and dg2 == digests[:k] and bool(torch.equal(d_back[: k * stride_in - (stride_in - chunk_bytes)], d_in[: k * stride_in - (stride_in - chunk_bytes)]))
+        del d_back
+        if not roundtrip:
+            raise SystemExit("LZ4 frames do not decode back to the input -- refusing to report a number")
+    res = {"elapsed": elapsed, "kernel_ms": statistics.mean(kernel_ms), "frame_bytes": sum(out_lens), "launches": launches,
+           "clocks": clocks, "roundtrip": roundtrip, "total_in": n_chunks * chunk_bytes,
+           "outputs": sample_outputs(torch, np, d_out, dst_off, out_lens, digests) if dump else None}
     ctx.close()
     del d_in, d_out
     torch.cuda.empty_cache()
@@ -440,7 +467,8 @@ def run_gpu(args):
 
     # ---- value: device-resident batch, CUDA events, MAX over ranks
     barrier()
-    r = device_resident_run(torch, native, dev, local, args.workload, n_chunks, chunk_bytes, rank, args.steps, args.warmup)
+    dump = bool(args.dump_outputs) and rank == 0
+    r = device_resident_run(torch, native, dev, local, args.workload, n_chunks, chunk_bytes, rank, args.steps, args.warmup, dump=dump)
     barrier()
     elapsed = max_over_ranks(r["elapsed"], dev)
     clocks, gpu_launches = r["clocks"], r["launches"]
@@ -567,7 +595,7 @@ def run_gpu(args):
     if do_c3:
         barrier()
         c3 = device_resident_run(torch, native, dev, local, "silesia", args.c3_chunks, 16 << 20, rank, max(2, args.steps // 2), 2,
-                                 sample_clocks=False, verify_decode=True)
+                                 sample_clocks=False, verify_decode=True, dump=dump)
         barrier()
         el3 = max_over_ranks(c3["elapsed"], dev)
         steps3 = max(2, args.steps // 2)
@@ -589,12 +617,20 @@ def run_gpu(args):
             cmd = [sys.executable, "-m", "skyplane_b200.harness", "--gpus", str(world), "--chunks", str(args.queue_chunks * world), "--chunk-mib",
                    str(args.chunk_mib), "--workload", args.workload if args.workload == "random" else "silesia", "--pool", "32", "--batch", "128", "--slots", "4"]
             env = {k: v for k, v in os.environ.items() if k not in ("RANK", "LOCAL_RANK", "WORLD_SIZE", "MASTER_ADDR", "MASTER_PORT")}
+            env["PYTHONDONTWRITEBYTECODE"] = "1"
             try:
                 out = subprocess.run(cmd, capture_output=True, text=True, timeout=240, cwd=str(ROOT), env=env)
                 queue_e2e = json.loads(out.stdout.strip().splitlines()[-1]) if out.returncode == 0 else {"error": out.stderr[-400:]}
             except Exception as e:  # a broken harness must not take the bench line down with it
                 queue_e2e = {"error": repr(e)}
         barrier()
+
+    if dump:
+        dump_dir = Path(args.dump_outputs)
+        dump_dir.mkdir(parents=True, exist_ok=True)
+        for prefix, rec in (("", r), ("config3_", c3 if do_c3 else None)):
+            for name, arr in ((rec or {}).get("outputs") or {}).items():
+                np.save(dump_dir / f"{prefix}{name}.npy", arr)
 
     if rank == 0:
         cfg = workload_config(args, world)
@@ -631,6 +667,7 @@ def main():
     ap.add_argument("--no-queue-e2e", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the last timed step's outputs as .npy files into DIR")
     args = ap.parse_args()
     if args.warmup < 3 and args.impl == "b200":
         print("note: timing rules ask for >= 3 warm-up steps", file=sys.stderr)
