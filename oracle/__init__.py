@@ -120,7 +120,9 @@ def lz4f_compress_indep(data) -> bytes:
 
 
 def lz4f_decode(frame, max_out: int | None = None, with_info: bool = False):
-    """Strict LZ4 frame decoder (what ``lz4.frame.decompress`` must accept). Raises OracleError."""
+    """Strict LZ4 frame decoder: rejects what ``lz4.frame.decompress`` rejects, and additionally enforces the block
+    format's end-of-block rules (last match >= 12 bytes before the block end, last 5 bytes literals) and offset != 0,
+    which liblz4 lets through in a few cases. Raises OracleError."""
     p, n, _k = _ro(frame)
     if max_out is None:
         mv = memoryview(frame).cast("B")

@@ -8,6 +8,9 @@
 //                 emits) decode fully in parallel; linked-block frames (what the reference's CPU sender emits)
 //                 decode block j after block j-1 of the same chunk (matches may reach into earlier output).
 // Every read and write is bounds-checked: a malformed frame yields an error status, never an out-of-range access.
+// It rejects what liblz4 rejects, and additionally enforces the block format's end-of-block rules (a match starts at
+// least 12 bytes before the end of its block, the last 5 bytes are literals) and offset != 0: liblz4 checks the former
+// against the room left in its 64 KiB block buffer rather than the block's real end, and lets offset 0 through.
 // The decoded size of block j is taken to be min(64 KiB, raw_len - j*64 KiB) -- true for liblz4 and for our
 // encoder (only the last block is short); anything else is reported as SKY_D_LAYOUT.
 #pragma once
@@ -150,7 +153,7 @@ __device__ __forceinline__ int32_t lz4_decode_block(const uint8_t *src, uint32_t
             } while (s == 255 && ml < (1u << 24));
         }
         ml += kMinMatch;
-        if (op + ml > oend) return kDecCorrupt;
+        if (op + kMfLimit > oend || op + ml + kLastLiterals > oend) return kDecCorrupt;  // end-of-block rules
         __syncwarp();  // the literals just written may be the match source
         warp_match_copy(out + op, offset, ml, lane);
         op += ml;
