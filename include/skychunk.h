@@ -67,7 +67,9 @@ extern "C" {
 typedef struct sky_ctx sky_ctx;
 
 SKY_API const char *sky_strerror(int code);
-SKY_API const char *sky_last_error(const sky_ctx *ctx); /* detail of the last SKY_E_CUDA on this ctx */
+/* Detail of the latest failed call on this ctx.  ctx = NULL: of the latest failed call on this thread that had no ctx
+ * (sky_ctx_create, the device queries, sky_pinned_alloc / sky_pinned_free, a NULL ctx argument). */
+SKY_API const char *sky_last_error(const sky_ctx *ctx);
 SKY_API int sky_abi_version(void);
 SKY_API int sky_device_count(int *count);
 /* PCI bus id ("0000:1b:00.0") of CUDA device `device` as the CUDA runtime orders devices (honours CUDA_VISIBLE_DEVICES,

@@ -294,12 +294,6 @@ __device__ __forceinline__ bool mbar_try_wait_hint(uint64_t *bar, uint32_t parit
                  : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity), "r"(ns) : "memory");
     return ok != 0;
 }
-__device__ __forceinline__ bool mbar_test_wait(uint64_t *bar, uint32_t parity) {  // never suspends
-    uint32_t ok;
-    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                 : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-    return ok != 0;
-}
 __device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
     while (!mbar_try_wait_hint(bar, parity, 20000u)) {}
 }

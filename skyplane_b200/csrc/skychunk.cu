@@ -24,6 +24,8 @@
 // There is NO CPU fallback anywhere in this file: without a CUDA device every entry point fails.
 
 #include <cuda_runtime.h>
+#include <inttypes.h>
+#include <stdarg.h>
 #include <stdint.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -53,14 +55,6 @@ constexpr int kThreads = kWarps * 32;
 #ifndef SKY_RING_EXTRA
 #define SKY_RING_EXTRA 2
 #endif
-#ifndef SKY_WAIT_NS
-#define SKY_WAIT_NS 0
-#endif
-#ifndef SKY_PACE_LEAD
-#define SKY_PACE_LEAD 0
-#endif
-constexpr uint32_t kWaitNs = SKY_WAIT_NS;       // 0: a waiting parser is parked by mbarrier.try_wait (measured best); else it sleeps, doubling up to this many ns
-constexpr uint32_t kPaceLead = SKY_PACE_LEAD;   // rows the compressor may run ahead of a chunk's MD5 lanes beyond the one they are in
 constexpr int kRing = kParsers + SKY_RING_EXTRA;       // segment slots between the prober and the parsers
 constexpr int kMd5WarpsPerCta = 4;        // digest CTAs run 4 MD5 groups (one per SM sub-partition), see sky_fused_kernel
 constexpr uint32_t kRingBytes = SKY_MD5_SLOTS * 2048;  // MD5 staging ring: slots x 64 B x 32 lanes
@@ -183,7 +177,7 @@ __device__ __forceinline__ void claim_block(const Params &p, BlockDesc *d, bool 
             for (;;) {
                 const uint32_t pr = ld_relaxed32(pw);
                 // pr: 0 = digest not started, 0xffffffff = finished, else 1 + rows consumed (64-bit compare: no wrap)
-                if (pr == 0 || (uint64_t)j + 1 <= (uint64_t)pr + lead + kPaceLead) break;
+                if (pr == 0 || (uint64_t)j + 1 <= (uint64_t)pr + lead) break;
                 __nanosleep(ns);
                 if (ns < 4096) ns <<= 1;
             }
@@ -360,15 +354,10 @@ __global__ void __launch_bounds__(kThreads, 2) sky_fused_kernel(const Params p) 
                 // (mbarrier.try_wait's hardware suspend ends at every barrier event in the CTA, a few dozen ns apart here, so the
                 // waiting loops are a quarter of the instructions issued -- but replacing them with timed sleeps gained
                 // nothing (r2_29: 115.9 vs 116.3 GB/s): the issue slots they take are not the ones the parsers lack.)
-                unsigned ns = 32;
-                while (!(kWaitNs ? mbar_test_wait(&ctl->full[si], ph) : mbar_try_wait_hint(&ctl->full[si], ph, 1000u))) {
+                while (!mbar_try_wait_hint(&ctl->full[si], ph, 1000u)) {
                     if (atomicAdd(const_cast<uint32_t *>(&ctl->block_end_seq), 0u) <= my_seq) {  // no such segment in this block: keep the claim
                         got = mbar_try_wait(&ctl->full[si], ph);
                         break;
-                    }
-                    if (kWaitNs) {
-                        __nanosleep(ns);
-                        if (ns < kWaitNs) ns <<= 1;
                     }
                 }
                 if (!got) break;
@@ -626,20 +615,13 @@ __global__ void __launch_bounds__(512, 1) sky_decode_kernel(const DecParams p) {
 }
 
 // ---- E2EE glue: describe one box per chunk once the frame lengths exist (they are only known on the device).
-// seal: msg = the chunk's frame (or, without LZ4, its raw bytes), box = box_base + (frame offset in the frame slab) + 64*i + 8,
-// so that box + 40 is 16-byte aligned; the nonce is copied in, out_len becomes the box length.
-__global__ void sky_box_setup_kernel(BoxChunk *bc, uint64_t *blk_base, const ChunkDesc *desc, uint32_t n, uint64_t *out_len,
-                                     const uint8_t *frame_slab, uint8_t *box_slab, const uint8_t *nonces, int use_frames) {
-    for (uint32_t i = threadIdx.x; i < n; i += blockDim.x) {
-        const ChunkDesc d = desc[i];
-        BoxChunk b;
-        b.box = box_slab + (d.dst - frame_slab) + 64ull * i + 8;
-        b.msg = use_frames ? d.dst : d.src;
-        b.len = use_frames ? out_len[i] : d.len;
-        for (int k = 0; k < 24; k++) b.box[k] = nonces[24ull * i + k];
-        bc[i] = b;
-        out_len[i] = b.len + kBoxOverhead;
-    }
+// Box i of a batch sits in the box slab at the offset of chunk i's frame in the frame slab + 64*i + 8: the box is 40 bytes
+// longer than its payload, and box + 40 (the ciphertext) is 16-byte aligned like the payload.
+__host__ __device__ inline uint64_t box_offset(uint64_t frame_off, uint32_t i) { return frame_off + 64ull * i + 8; }
+
+// Both setup kernels end here: blk_base[i] = the 64-byte stream blocks of the boxes before box i (block 0's second half
+// covers message bytes [0, 32), hence len + 32), blk_base[n] = their total; sky_box_xor_kernel splits its work by it.
+__device__ void box_block_prefix(const BoxChunk *bc, uint64_t *blk_base, uint32_t n) {
     __syncthreads();
     if (threadIdx.x == 0) {
         uint64_t acc = 0;
@@ -650,25 +632,33 @@ __global__ void sky_box_setup_kernel(BoxChunk *bc, uint64_t *blk_base, const Chu
         blk_base[n] = acc;
     }
 }
-// open: the boxes were copied to box_slab (box i at box_off[i] + 8); the plaintext frame goes to frame_slab + frame_off[i].
-__global__ void sky_box_open_setup_kernel(BoxChunk *bc, uint64_t *blk_base, uint32_t n, const uint64_t *box_off, const uint64_t *box_len,
+
+// seal: msg = the chunk's frame (or, without LZ4, its raw bytes); the nonce is copied in, out_len becomes the box length.
+__global__ void sky_box_setup_kernel(BoxChunk *bc, uint64_t *blk_base, const ChunkDesc *desc, uint32_t n, uint64_t *out_len,
+                                     const uint8_t *frame_slab, uint8_t *box_slab, const uint8_t *nonces, int use_frames) {
+    for (uint32_t i = threadIdx.x; i < n; i += blockDim.x) {
+        const ChunkDesc d = desc[i];
+        BoxChunk b;
+        b.box = box_slab + box_offset(d.dst - frame_slab, i);
+        b.msg = use_frames ? d.dst : d.src;
+        b.len = use_frames ? out_len[i] : d.len;
+        for (int k = 0; k < 24; k++) b.box[k] = nonces[24ull * i + k];
+        bc[i] = b;
+        out_len[i] = b.len + kBoxOverhead;
+    }
+    box_block_prefix(bc, blk_base, n);
+}
+// open: the boxes were copied into box_slab; the plaintext frame goes to frame_slab + frame_off[i].
+__global__ void sky_box_open_setup_kernel(BoxChunk *bc, uint64_t *blk_base, uint32_t n, const uint64_t *box_len,
                                           const uint64_t *frame_off, uint8_t *frame_slab, uint8_t *box_slab) {
     for (uint32_t i = threadIdx.x; i < n; i += blockDim.x) {
         BoxChunk b;
-        b.box = box_slab + box_off[i] + 8;
+        b.box = box_slab + box_offset(frame_off[i], i);
         b.msg = frame_slab + frame_off[i];
         b.len = box_len[i] >= (uint64_t)kBoxOverhead ? box_len[i] - kBoxOverhead : 0;
         bc[i] = b;
     }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        uint64_t acc = 0;
-        for (uint32_t i = 0; i < n; i++) {
-            blk_base[i] = acc;
-            acc += (bc[i].len + 32 + 63) / 64;
-        }
-        blk_base[n] = acc;
-    }
+    box_block_prefix(bc, blk_base, n);
 }
 
 }  // namespace sky
@@ -676,38 +666,60 @@ __global__ void sky_box_open_setup_kernel(BoxChunk *bc, uint64_t *blk_base, uint
 // ======================================================================================= host side
 using namespace sky;
 
+// One allocation that frees itself: device or pinned host memory, an event or a stream.  Every allocation a slot or the
+// ctx makes is held by one of these members, so a half-built ctx is torn down by the same destructors as a finished one.
+// put() frees what the handle held and gives the allocating call the pointer to fill.
+template <class T, cudaError_t (*Free)(void *)>
+struct Owned {
+    T *p = nullptr;
+    Owned() = default;
+    Owned(Owned &&o) noexcept : p(o.p) { o.p = nullptr; }
+    ~Owned() { reset(); }
+    void reset() { if (p) Free(p); p = nullptr; }
+    T **put() { reset(); return &p; }
+    operator T *() const { return p; }
+};
+inline cudaError_t destroy_event(void *e) { return cudaEventDestroy(static_cast<cudaEvent_t>(e)); }
+inline cudaError_t destroy_stream(void *s) { return cudaStreamDestroy(static_cast<cudaStream_t>(s)); }
+template <class T> using Dev = Owned<T, cudaFree>;
+template <class T> using Pinned = Owned<T, cudaFreeHost>;
+using Event = Owned<CUevent_st, destroy_event>;
+using Stream = Owned<CUstream_st, destroy_stream>;
+
 struct Slot {
-    cudaStream_t stream = nullptr;
-    uint8_t *d_in = nullptr, *d_out = nullptr;
-    cudaEvent_t ev_k0 = nullptr, ev_k1 = nullptr, ev_res = nullptr;  // kernel start / end, results (sizes+digests) on host
+    Stream stream;
+    Dev<uint8_t> d_in, d_out;  // host path (n_slots > 0): input slab, frame slab
+    Event ev_k0, ev_k1;        // start / end of the slot's kernels (kernel_ms): the fused kernel, or frame index + decode
+    Event ev_res;              // results (sizes + digests) are on the host
+    Event ev_h2d, ev_d2h;      // input landed (on ctx->st_h2d) / frames landed (on ctx->st_d2h)
+    Event ev_h0, ev_d0, ev_d1; // SKYCHUNK_TRACE only: H2D start, D2H start / end
     bool d2h_issued = false;
-    cudaEvent_t ev_h0 = nullptr, ev_d0 = nullptr, ev_d1 = nullptr;  // SKYCHUNK_TRACE only: H2D start, D2H start / end
-    // per-batch metadata (device + pinned host mirrors)
-    ChunkDesc *h_desc = nullptr, *d_desc = nullptr;
-    uint32_t *h_order = nullptr, *d_order = nullptr;
-    uint64_t *h_chain = nullptr, *d_chain = nullptr;
-    uint32_t *d_freed = nullptr, *d_progress = nullptr;
+    // per-batch metadata (pinned host mirrors + device arrays)
+    Pinned<ChunkDesc> h_desc; Dev<ChunkDesc> d_desc;
+    Pinned<uint32_t> h_order; Dev<uint32_t> d_order;
+    Pinned<uint64_t> h_chain; Dev<uint64_t> d_chain;
+    Dev<uint32_t> d_progress;
     // results live in MAPPED pinned host memory: the kernel stores sizes / digests straight over PCIe, so no small
     // device->host copies sit in a copy-engine queue behind multi-GiB frame copies
-    uint64_t *h_outlen = nullptr, *d_outlen = nullptr;  // same allocation, host / device view
-    uint8_t *h_md5 = nullptr, *d_md5 = nullptr;
-    cudaEvent_t ev_h2d = nullptr, ev_d2h = nullptr;  // input landed (on ctx->st_h2d) / frames landed (on ctx->st_d2h)
-    uint32_t *d_counters = nullptr;
-    uint8_t *d_scratch = nullptr;  // compress scratch: kScratchBytes per CTA of the grid (kernels of different slots overlap)
+    Pinned<uint64_t> h_outlen; uint64_t *d_outlen = nullptr;  // same allocation, host / device view
+    Pinned<uint8_t> h_md5; uint8_t *d_md5 = nullptr;
+    Dev<uint32_t> d_counters;
+    Dev<uint8_t> d_scratch;  // compress scratch: kScratchBytes per CTA of the grid (kernels of different slots overlap)
     // receiver side
-    DecChunk *h_dchunks = nullptr, *d_dchunks = nullptr;
-    DecBlock *d_dblocks = nullptr;
-    uint32_t *d_blkdone = nullptr;
+    Pinned<DecChunk> h_dchunks; Dev<DecChunk> d_dchunks;
+    Dev<DecBlock> d_dblocks;      // block table, dblocks_cap entries
+    Dev<uint32_t> d_block_flags;  // per block: 1 once decoded (gates the MD5 lanes), dblocks_cap entries
     uint64_t dblocks_cap = 0;
-    int32_t *h_dstatus = nullptr, *d_dstatus = nullptr;  // pinned host mirror / device array
+    Dev<uint32_t> d_blocks_done;  // per chunk: leading blocks decoded (linked frames decode in order)
+    Pinned<int32_t> h_dstatus; Dev<int32_t> d_dstatus;
     // E2EE (allocated when a key is set): box slab, per-chunk box descriptors, stream-block prefix, subkeys, nonces
-    uint8_t *d_box = nullptr;
-    BoxChunk *d_bchunks = nullptr;
-    uint64_t *d_blkbase = nullptr;
-    uint32_t *d_sub = nullptr;
-    uint8_t *h_nonce = nullptr, *d_nonce = nullptr;
-    uint64_t *h_boxmeta = nullptr, *d_boxmeta = nullptr;  // open side: box_off | box_len | frame_off (3 x n)
-    int32_t *h_bstatus = nullptr, *d_bstatus = nullptr;
+    Dev<uint8_t> d_box;
+    Dev<BoxChunk> d_bchunks;
+    Dev<uint64_t> d_blkbase;
+    Dev<uint32_t> d_sub;
+    Pinned<uint8_t> h_nonce; Dev<uint8_t> d_nonce;
+    Pinned<uint64_t> h_boxmeta; Dev<uint64_t> d_boxmeta;  // open side: box_len | frame_off (2 x n)
+    Pinned<int32_t> h_bstatus; Dev<int32_t> d_bstatus;
     uint32_t flags = 0;
     // in-flight ticket
     bool busy = false;
@@ -720,35 +732,89 @@ struct Slot {
 struct sky_ctx {
     int device = 0;
     int sm_count = 0;
-    uint64_t max_bytes = 0;
     uint32_t max_chunks = 0;
     uint64_t in_cap = 0, out_cap = 0;
     std::vector<Slot> slots;  // slots[0] doubles as the metadata holder for sky_process_device
     uint64_t next_ticket = 1;
     uint64_t launches = 0;
-    std::string err;
+    std::string err;  // sky_last_error
     // Host path: every slot's input copies go FIFO through one H2D stream and every frame copy through one D2H
     // stream, so the two directions use different copy engines and batch k's frames leave while batch k+1's
     // input arrives (per-slot streams put both directions of all slots into one in-order engine queue).
-    cudaStream_t st_h2d = nullptr, st_d2h = nullptr;
-    uint8_t *d_key = nullptr;  // 32-byte SecretBox key (null: E2EE off)
-    bool trace = false;           // SKYCHUNK_TRACE=1: print per-batch device timeline to stderr
-    cudaEvent_t ev_base = nullptr;
+    Stream st_h2d, st_d2h;
+    Dev<uint8_t> d_key;  // 32-byte SecretBox key (null: E2EE off)
+    bool trace = false;  // SKYCHUNK_TRACE=1: print per-batch device timeline to stderr
+    Event ev_base;
+    // a copy on the shared streams may still read a slot's slabs: wait for all of them before the members free themselves
+    ~sky_ctx() {
+        cudaSetDevice(device);
+        for (auto &s : slots)
+            if (s.stream) cudaStreamSynchronize(s.stream);
+        if (st_h2d) cudaStreamSynchronize(st_h2d);
+        if (st_d2h) cudaStreamSynchronize(st_d2h);
+    }
 };
 
-static thread_local std::string g_err;
+static thread_local std::string g_err;  // sky_last_error(NULL)
 
-#define CK(ctx, call)                                                                      \
-    do {                                                                                   \
-        cudaError_t e_ = (call);                                                           \
-        if (e_ != cudaSuccess) {                                                           \
-            char b_[512];                                                                  \
-            snprintf(b_, sizeof b_, "%s -> %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); \
-            if (ctx) (ctx)->err = b_;                                                      \
-            g_err = b_;                                                                    \
-            return SKY_E_CUDA;                                                             \
-        }                                                                                  \
+// Every failing return of an entry point goes through here: the detail goes to the ctx, or to the calling thread when
+// there is none, so sky_last_error always describes the latest failure.
+__attribute__((format(printf, 3, 4))) static int fail(sky_ctx *ctx, int rc, const char *fmt, ...) {
+    char b[512];
+    va_list ap;
+    va_start(ap, fmt);
+    vsnprintf(b, sizeof b, fmt, ap);
+    va_end(ap);
+    (ctx ? ctx->err : g_err) = b;
+    return rc;
+}
+
+#define CK(ctx, call)                                                                                                   \
+    do {                                                                                                                \
+        const cudaError_t e_ = (call);                                                                                  \
+        if (e_ != cudaSuccess) return fail(ctx, SKY_E_CUDA, "%s -> %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); \
     } while (0)
+
+static uint64_t round16(uint64_t x) { return (x + 15) & ~15ull; }
+
+// Offsets of n regions of len(i) bytes packed back to back into a slab, each at a 16-byte aligned offset; end = bytes used.
+template <class Len>
+static std::vector<uint64_t> pack16(uint32_t n, Len len, uint64_t &end) {
+    std::vector<uint64_t> off(n);
+    end = 0;
+    for (uint32_t i = 0; i < n; i++) {
+        off[i] = end;
+        end += round16(len(i));
+    }
+    return off;
+}
+
+// Stage flags 0 mean LZ4 + MD5.
+static uint32_t with_default_stages(uint32_t flags) {
+    return (flags & (SKY_F_LZ4 | SKY_F_MD5)) ? flags : flags | SKY_F_LZ4 | SKY_F_MD5;
+}
+
+static uint64_t nblocks(uint64_t len) { return (len + kBlock - 1) / kBlock; }
+// 64 KiB block rows of a batch: max(1, blocks of its longest chunk).  The kernels hold a block index in 24 bits (the
+// fused kernel's OFF word) and number their work items (rows x n) in 32.
+static int block_rows(sky_ctx *ctx, uint32_t n, const uint64_t *len, uint32_t *rows) {
+    uint64_t r = 1;
+    for (uint32_t i = 0; i < n; i++) r = std::max(r, nblocks(len[i]));
+    if (r >= (1ull << 24) || r * n >= 0xffffffffull)
+        return fail(ctx, SKY_E_CAPACITY, "%" PRIu64 " block rows x %u chunks exceed the kernels' block and work counters", r, n);
+    *rows = (uint32_t)r;
+    return SKY_OK;
+}
+
+// MD5 lane assignment: chunk indices, longest chunk first so a warp's 32 lanes carry similar lengths, padded with
+// 0xffffffff to whole groups of 32.  Returns the number of groups.
+static uint32_t md5_lane_order(uint32_t *order, uint32_t n, const uint64_t *len) {
+    const uint32_t ng = (n + 31) / 32;
+    std::iota(order, order + n, 0u);
+    std::stable_sort(order, order + n, [&](uint32_t a, uint32_t b) { return len[a] > len[b]; });
+    std::fill(order + n, order + ng * 32, 0xffffffffu);
+    return ng;
+}
 
 extern "C" {
 
@@ -771,25 +837,21 @@ const char *sky_last_error(const sky_ctx *ctx) { return ctx ? ctx->err.c_str() :
 int sky_abi_version(void) { return SKY_ABI_VERSION; }
 
 int sky_device_count(int *count) {
-    if (!count) return SKY_E_INVALID;
+    if (!count) return fail(nullptr, SKY_E_INVALID, "count is NULL");
     int n = 0;
-    cudaError_t e = cudaGetDeviceCount(&n);
+    const cudaError_t e = cudaGetDeviceCount(&n);
     if (e != cudaSuccess || n <= 0) {
         *count = 0;
-        g_err = cudaGetErrorString(e);
-        return SKY_E_NOGPU;
+        return fail(nullptr, SKY_E_NOGPU, "cudaGetDeviceCount -> %s", cudaGetErrorString(e));
     }
     *count = n;
     return SKY_OK;
 }
 
 int sky_device_pci_bus_id(int device, char *buf, int len) {
-    if (!buf || len < 16) return SKY_E_INVALID;
-    cudaError_t e = cudaDeviceGetPCIBusId(buf, len, device);
-    if (e != cudaSuccess) {
-        g_err = cudaGetErrorString(e);
-        return e == cudaErrorInvalidDevice ? SKY_E_INVALID : SKY_E_NOGPU;
-    }
+    if (!buf || len < 16) return fail(nullptr, SKY_E_INVALID, "buf is NULL or len < 16");
+    const cudaError_t e = cudaDeviceGetPCIBusId(buf, len, device);
+    if (e != cudaSuccess) return fail(nullptr, e == cudaErrorInvalidDevice ? SKY_E_INVALID : SKY_E_NOGPU, "%s", cudaGetErrorString(e));
     return SKY_OK;
 }
 
@@ -808,177 +870,138 @@ uint64_t sky_frame_bound(uint64_t n) {
     return 15 + n + 4 * ((n + kBlock - 1) / kBlock) + 4;
 }
 
-static uint64_t round16(uint64_t x) { return (x + 15) & ~15ull; }
-
-static int alloc_meta(sky_ctx *ctx, Slot &s, uint32_t max_chunks) {
-    const size_t nc = max_chunks, ng = (nc + 31) / 32 * 32;
-    CK(ctx, cudaMallocHost(&s.h_desc, nc * sizeof(ChunkDesc)));
-    CK(ctx, cudaMallocHost(&s.h_order, ng * sizeof(uint32_t)));
-    CK(ctx, cudaMallocHost(&s.h_chain, nc * sizeof(uint64_t)));
-    CK(ctx, cudaHostAlloc(&s.h_outlen, nc * sizeof(uint64_t), cudaHostAllocMapped | cudaHostAllocPortable));
-    CK(ctx, cudaHostAlloc(&s.h_md5, nc * 16, cudaHostAllocMapped | cudaHostAllocPortable));
+// Everything a slot needs for any batch: metadata, results, decode arrays, stream and events (+ the slabs on the host path).
+static int alloc_slot(sky_ctx *ctx, Slot &s, bool slabs) {
+    const size_t nc = ctx->max_chunks, ng = (nc + 31) / 32 * 32;
+    CK(ctx, cudaMallocHost(s.h_desc.put(), nc * sizeof(ChunkDesc)));
+    CK(ctx, cudaMallocHost(s.h_order.put(), ng * sizeof(uint32_t)));
+    CK(ctx, cudaMallocHost(s.h_chain.put(), nc * sizeof(uint64_t)));
+    CK(ctx, cudaHostAlloc(s.h_outlen.put(), nc * sizeof(uint64_t), cudaHostAllocMapped | cudaHostAllocPortable));
+    CK(ctx, cudaHostAlloc(s.h_md5.put(), nc * 16, cudaHostAllocMapped | cudaHostAllocPortable));
     CK(ctx, cudaHostGetDevicePointer(&s.d_outlen, s.h_outlen, 0));
     CK(ctx, cudaHostGetDevicePointer(&s.d_md5, s.h_md5, 0));
-    CK(ctx, cudaEventCreateWithFlags(&s.ev_h2d, cudaEventDisableTiming));
-    CK(ctx, cudaEventCreateWithFlags(&s.ev_d2h, cudaEventDisableTiming));
-    CK(ctx, cudaMalloc(&s.d_desc, nc * sizeof(ChunkDesc)));
-    CK(ctx, cudaMalloc(&s.d_order, ng * sizeof(uint32_t)));
-    CK(ctx, cudaMalloc(&s.d_chain, nc * sizeof(uint64_t)));
-    CK(ctx, cudaMalloc(&s.d_counters, 64));
-    CK(ctx, cudaMalloc(&s.d_scratch, (size_t)ctx->sm_count * kCtasPerSm * kScratchBytes));
-    CK(ctx, cudaMallocHost(&s.h_dchunks, nc * sizeof(DecChunk)));
-    CK(ctx, cudaMalloc(&s.d_dchunks, nc * sizeof(DecChunk)));
-    CK(ctx, cudaMallocHost(&s.h_dstatus, nc * sizeof(int32_t)));
-    CK(ctx, cudaMalloc(&s.d_dstatus, nc * sizeof(int32_t)));
-    CK(ctx, cudaMalloc(&s.d_freed, nc * sizeof(uint32_t)));
-    CK(ctx, cudaMalloc(&s.d_progress, (ng / 32 + 1) * sizeof(uint32_t)));
-    CK(ctx, cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking));
-    CK(ctx, cudaEventCreate(&s.ev_k0));
-    CK(ctx, cudaEventCreate(&s.ev_k1));
-    CK(ctx, cudaEventCreate(&s.ev_res));
-    CK(ctx, cudaEventCreate(&s.ev_h0));
-    CK(ctx, cudaEventCreate(&s.ev_d0));
-    CK(ctx, cudaEventCreate(&s.ev_d1));
+    CK(ctx, cudaEventCreateWithFlags(s.ev_h2d.put(), cudaEventDisableTiming));
+    CK(ctx, cudaEventCreateWithFlags(s.ev_d2h.put(), cudaEventDisableTiming));
+    CK(ctx, cudaMalloc(s.d_desc.put(), nc * sizeof(ChunkDesc)));
+    CK(ctx, cudaMalloc(s.d_order.put(), ng * sizeof(uint32_t)));
+    CK(ctx, cudaMalloc(s.d_chain.put(), nc * sizeof(uint64_t)));
+    CK(ctx, cudaMalloc(s.d_counters.put(), 64));
+    CK(ctx, cudaMalloc(s.d_scratch.put(), (size_t)ctx->sm_count * kCtasPerSm * kScratchBytes));
+    CK(ctx, cudaMallocHost(s.h_dchunks.put(), nc * sizeof(DecChunk)));
+    CK(ctx, cudaMalloc(s.d_dchunks.put(), nc * sizeof(DecChunk)));
+    CK(ctx, cudaMallocHost(s.h_dstatus.put(), nc * sizeof(int32_t)));
+    CK(ctx, cudaMalloc(s.d_dstatus.put(), nc * sizeof(int32_t)));
+    CK(ctx, cudaMalloc(s.d_blocks_done.put(), nc * sizeof(uint32_t)));
+    CK(ctx, cudaMalloc(s.d_progress.put(), (ng / 32 + 1) * sizeof(uint32_t)));
+    CK(ctx, cudaStreamCreateWithFlags(s.stream.put(), cudaStreamNonBlocking));
+    CK(ctx, cudaEventCreate(s.ev_k0.put()));
+    CK(ctx, cudaEventCreate(s.ev_k1.put()));
+    CK(ctx, cudaEventCreate(s.ev_res.put()));
+    CK(ctx, cudaEventCreate(s.ev_h0.put()));
+    CK(ctx, cudaEventCreate(s.ev_d0.put()));
+    CK(ctx, cudaEventCreate(s.ev_d1.put()));
+    if (slabs) {
+        cudaError_t e = cudaMalloc(s.d_in.put(), ctx->in_cap);
+        if (e == cudaSuccess) e = cudaMalloc(s.d_out.put(), ctx->out_cap);
+        if (e != cudaSuccess) return fail(ctx, SKY_E_NOMEM, "cudaMalloc(slab) -> %s", cudaGetErrorString(e));
+    }
     return SKY_OK;
 }
 
-static void free_slot(Slot &s) {
-    if (s.stream) cudaStreamSynchronize(s.stream);
-    cudaFreeHost(s.h_desc); cudaFreeHost(s.h_order); cudaFreeHost(s.h_chain); cudaFreeHost(s.h_outlen); cudaFreeHost(s.h_md5);
-    cudaFree(s.d_desc); cudaFree(s.d_order); cudaFree(s.d_chain); cudaFree(s.d_counters);
-    cudaFreeHost(s.h_dchunks); cudaFree(s.d_dchunks); cudaFree(s.d_dblocks); cudaFree(s.d_blkdone); cudaFreeHost(s.h_dstatus); cudaFree(s.d_dstatus); cudaFree(s.d_freed); cudaFree(s.d_progress);
-    cudaFree(s.d_in); cudaFree(s.d_out); cudaFree(s.d_scratch);
-    cudaFree(s.d_box); cudaFree(s.d_bchunks); cudaFree(s.d_blkbase); cudaFree(s.d_sub); cudaFree(s.d_nonce); cudaFreeHost(s.h_nonce);
-    cudaFree(s.d_boxmeta); cudaFreeHost(s.h_boxmeta); cudaFree(s.d_bstatus); cudaFreeHost(s.h_bstatus);
-    if (s.ev_k0) cudaEventDestroy(s.ev_k0);
-    if (s.ev_k1) cudaEventDestroy(s.ev_k1);
-    if (s.ev_res) cudaEventDestroy(s.ev_res);
-    if (s.ev_h2d) cudaEventDestroy(s.ev_h2d);
-    if (s.ev_d2h) cudaEventDestroy(s.ev_d2h);
-    if (s.ev_h0) cudaEventDestroy(s.ev_h0);
-    if (s.ev_d0) cudaEventDestroy(s.ev_d0);
-    if (s.ev_d1) cudaEventDestroy(s.ev_d1);
-    if (s.stream) cudaStreamDestroy(s.stream);
-    s = Slot();
-}
-
-int sky_ctx_create(int device, uint64_t max_batch_bytes, uint32_t max_chunks, uint32_t n_slots, sky_ctx **out) {
-    if (!out || max_chunks == 0) return SKY_E_INVALID;
-    *out = nullptr;
-    int ndev = 0;
-    if (sky_device_count(&ndev) != SKY_OK) return SKY_E_NOGPU;
-    if (device < 0 || device >= ndev) return SKY_E_INVALID;
-    sky_ctx *ctx = new (std::nothrow) sky_ctx();
-    if (!ctx) return SKY_E_NOMEM;
-    ctx->device = device;
-    ctx->max_bytes = max_batch_bytes;
-    ctx->max_chunks = max_chunks;
-    auto fail = [&](int rc) {
-        g_err = ctx->err;
-        for (auto &s : ctx->slots) free_slot(s);
-        if (ctx->st_h2d) cudaStreamDestroy(ctx->st_h2d);
-        if (ctx->st_d2h) cudaStreamDestroy(ctx->st_d2h);
-        delete ctx;
-        return rc;
-    };
-    cudaError_t e = cudaSetDevice(device);
-    if (e != cudaSuccess) { ctx->err = cudaGetErrorString(e); return fail(SKY_E_CUDA); }
+static int init_ctx(sky_ctx *ctx, uint64_t max_batch_bytes, uint32_t n_slots) {
+    CK(ctx, cudaSetDevice(ctx->device));
     cudaDeviceProp prop;
-    e = cudaGetDeviceProperties(&prop, device);
-    if (e != cudaSuccess) { ctx->err = cudaGetErrorString(e); return fail(SKY_E_CUDA); }
+    CK(ctx, cudaGetDeviceProperties(&prop, ctx->device));
     ctx->sm_count = prop.multiProcessorCount;
-    e = cudaFuncSetAttribute(sky_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes);
+    cudaError_t e = cudaFuncSetAttribute(sky_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(sky_fused_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-    if (e != cudaSuccess) {
-        ctx->err = std::string("cudaFuncSetAttribute(smem): ") + cudaGetErrorString(e) + " (built for sm_100a only)";
-        return fail(SKY_E_CUDA);
-    }
-    const uint32_t ns = n_slots ? n_slots : 1;
-    ctx->slots.resize(ns);
+    if (e != cudaSuccess) return fail(ctx, SKY_E_CUDA, "cudaFuncSetAttribute(smem) -> %s (built for sm_100a only)", cudaGetErrorString(e));
     // every chunk is placed at a 16-byte aligned offset; frames need bound(len) each
-    ctx->in_cap = round16(max_batch_bytes) + 16ull * max_chunks + 256;
-    ctx->out_cap = max_batch_bytes + (uint64_t)max_chunks * (64 + 4 * 2) + 4 * (max_batch_bytes / kBlock + 1) + 256;
-    for (uint32_t i = 0; i < ns; i++) {
-        int rc = alloc_meta(ctx, ctx->slots[i], max_chunks);
-        if (rc != SKY_OK) return fail(rc);
-        if (n_slots) {
-            e = cudaMalloc(&ctx->slots[i].d_in, ctx->in_cap);
-            if (e == cudaSuccess) e = cudaMalloc(&ctx->slots[i].d_out, ctx->out_cap);
-            if (e != cudaSuccess) { ctx->err = std::string("cudaMalloc(slab): ") + cudaGetErrorString(e); return fail(SKY_E_NOMEM); }
-        }
-    }
+    const uint64_t max_chunks = ctx->max_chunks;
+    ctx->in_cap = round16(max_batch_bytes) + 16 * max_chunks + 256;
+    ctx->out_cap = max_batch_bytes + max_chunks * (64 + 4 * 2) + 4 * (max_batch_bytes / kBlock + 1) + 256;
+    ctx->slots.resize(n_slots ? n_slots : 1);
+    for (auto &s : ctx->slots)
+        if (int rc = alloc_slot(ctx, s, n_slots != 0)) return rc;
     if (n_slots) {
-        e = cudaStreamCreateWithFlags(&ctx->st_h2d, cudaStreamNonBlocking);
-        if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&ctx->st_d2h, cudaStreamNonBlocking);
-        if (e != cudaSuccess) { ctx->err = cudaGetErrorString(e); return fail(SKY_E_CUDA); }
+        CK(ctx, cudaStreamCreateWithFlags(ctx->st_h2d.put(), cudaStreamNonBlocking));
+        CK(ctx, cudaStreamCreateWithFlags(ctx->st_d2h.put(), cudaStreamNonBlocking));
     }
     ctx->trace = getenv("SKYCHUNK_TRACE") != nullptr;
     if (ctx->trace) {
-        cudaEventCreate(&ctx->ev_base);
-        cudaEventRecord(ctx->ev_base, ctx->slots[0].stream);
+        CK(ctx, cudaEventCreate(ctx->ev_base.put()));
+        CK(ctx, cudaEventRecord(ctx->ev_base, ctx->slots[0].stream));
+    }
+    return SKY_OK;
+}
+
+int sky_ctx_create(int device, uint64_t max_batch_bytes, uint32_t max_chunks, uint32_t n_slots, sky_ctx **out) {
+    if (!out || max_chunks == 0) return fail(nullptr, SKY_E_INVALID, "out is NULL or max_chunks == 0");
+    *out = nullptr;
+    int ndev = 0;
+    if (int rc = sky_device_count(&ndev)) return rc;
+    if (device < 0 || device >= ndev) return fail(nullptr, SKY_E_INVALID, "device %d of %d", device, ndev);
+    sky_ctx *ctx = new (std::nothrow) sky_ctx();
+    if (!ctx) return fail(nullptr, SKY_E_NOMEM, "new sky_ctx");
+    ctx->device = device;
+    ctx->max_chunks = max_chunks;
+    if (int rc = init_ctx(ctx, max_batch_bytes, n_slots)) {
+        g_err = ctx->err;  // this ctx is never handed out
+        delete ctx;
+        return rc;
     }
     *out = ctx;
     return SKY_OK;
 }
 
 int sky_ctx_destroy(sky_ctx *ctx) {
-    if (!ctx) return SKY_E_INVALID;
-    cudaSetDevice(ctx->device);
-    for (auto &s : ctx->slots) free_slot(s);
-    if (ctx->st_h2d) { cudaStreamSynchronize(ctx->st_h2d); cudaStreamDestroy(ctx->st_h2d); }
-    if (ctx->st_d2h) { cudaStreamSynchronize(ctx->st_d2h); cudaStreamDestroy(ctx->st_d2h); }
-    if (ctx->ev_base) cudaEventDestroy(ctx->ev_base);
-    cudaFree(ctx->d_key);
+    if (!ctx) return fail(ctx, SKY_E_INVALID, "ctx is NULL");
     delete ctx;
     return SKY_OK;
 }
 
 void *sky_pinned_alloc(uint64_t bytes) {
     void *p = nullptr;
-    cudaError_t e = cudaHostAlloc(&p, bytes ? bytes : 1, cudaHostAllocPortable);
-    if (e != cudaSuccess) {
-        g_err = cudaGetErrorString(e);
-        return nullptr;
-    }
-    return p;
+    const cudaError_t e = cudaHostAlloc(&p, bytes ? bytes : 1, cudaHostAllocPortable);
+    if (e == cudaSuccess) return p;
+    fail(nullptr, SKY_E_NOMEM, "cudaHostAlloc(%" PRIu64 ") -> %s", bytes, cudaGetErrorString(e));
+    return nullptr;
 }
 int sky_pinned_free(void *p) {
-    if (!p) return SKY_OK;
-    return cudaFreeHost(p) == cudaSuccess ? SKY_OK : SKY_E_CUDA;
+    if (p) CK(nullptr, cudaFreeHost(p));
+    return SKY_OK;
 }
 
 uint64_t sky_box_bound(uint64_t n) { return sky_frame_bound(n) + kBoxOverhead; }
 
+// E2EE arrays of a slot, made once (d_box last: a partly failed earlier attempt is made again).
 static int alloc_box(sky_ctx *ctx, Slot &s) {
     if (s.d_box) return SKY_OK;
     const size_t nc = ctx->max_chunks;
-    CK(ctx, cudaMalloc(&s.d_box, ctx->out_cap + 64 * nc + 256));
-    CK(ctx, cudaMalloc(&s.d_bchunks, nc * sizeof(BoxChunk)));
-    CK(ctx, cudaMalloc(&s.d_blkbase, (nc + 1) * sizeof(uint64_t)));
-    CK(ctx, cudaMalloc(&s.d_sub, nc * 16 * sizeof(uint32_t)));
-    CK(ctx, cudaMalloc(&s.d_nonce, nc * 24));
-    CK(ctx, cudaMallocHost(&s.h_nonce, nc * 24));
-    CK(ctx, cudaMalloc(&s.d_boxmeta, 3 * nc * sizeof(uint64_t)));
-    CK(ctx, cudaMallocHost(&s.h_boxmeta, 3 * nc * sizeof(uint64_t)));
-    CK(ctx, cudaMalloc(&s.d_bstatus, nc * sizeof(int32_t)));
-    CK(ctx, cudaMallocHost(&s.h_bstatus, nc * sizeof(int32_t)));
+    CK(ctx, cudaMalloc(s.d_bchunks.put(), nc * sizeof(BoxChunk)));
+    CK(ctx, cudaMalloc(s.d_blkbase.put(), (nc + 1) * sizeof(uint64_t)));
+    CK(ctx, cudaMalloc(s.d_sub.put(), nc * 16 * sizeof(uint32_t)));
+    CK(ctx, cudaMalloc(s.d_nonce.put(), nc * 24));
+    CK(ctx, cudaMallocHost(s.h_nonce.put(), nc * 24));
+    CK(ctx, cudaMalloc(s.d_boxmeta.put(), 2 * nc * sizeof(uint64_t)));
+    CK(ctx, cudaMallocHost(s.h_boxmeta.put(), 2 * nc * sizeof(uint64_t)));
+    CK(ctx, cudaMalloc(s.d_bstatus.put(), nc * sizeof(int32_t)));
+    CK(ctx, cudaMallocHost(s.h_bstatus.put(), nc * sizeof(int32_t)));
+    CK(ctx, cudaMalloc(s.d_box.put(), ctx->out_cap + 64 * nc + 256));
     return SKY_OK;
 }
 
 int sky_set_e2ee_key(sky_ctx *ctx, const uint8_t *key32) {
-    if (!ctx) return SKY_E_INVALID;
+    if (!ctx) return fail(ctx, SKY_E_INVALID, "ctx is NULL");
     CK(ctx, cudaSetDevice(ctx->device));
     if (!key32) {
-        cudaFree(ctx->d_key);
-        ctx->d_key = nullptr;
+        ctx->d_key.reset();
         return SKY_OK;
     }
-    if (!ctx->d_key) CK(ctx, cudaMalloc(&ctx->d_key, 32));
+    if (!ctx->d_key) CK(ctx, cudaMalloc(ctx->d_key.put(), 32));
     CK(ctx, cudaMemcpy(ctx->d_key, key32, 32, cudaMemcpyHostToDevice));
-    for (auto &s : ctx->slots) {
-        int rc = alloc_box(ctx, s);
-        if (rc != SKY_OK) return rc;
-    }
+    for (auto &s : ctx->slots)
+        if (int rc = alloc_box(ctx, s)) return rc;
     return SKY_OK;
 }
 
@@ -1002,26 +1025,17 @@ static int launch_seal(sky_ctx *ctx, Slot &s, cudaStream_t st, uint32_t n, uint8
 // never queued behind another batch's frame copies); `st`: the stream the kernel runs on.
 static int launch_batch(sky_ctx *ctx, Slot &s, cudaStream_t st, cudaStream_t meta_st, uint32_t n, const uint8_t *d_src,
                         const uint64_t *src_off, const uint64_t *src_len, uint8_t *d_dst, const uint64_t *dst_off, uint32_t flags) {
-    if ((flags & (SKY_F_LZ4 | SKY_F_MD5)) == 0) flags |= SKY_F_LZ4 | SKY_F_MD5;
-    uint32_t rows = 1;
+    uint32_t rows;
+    if (int rc = block_rows(ctx, n, src_len, &rows)) return rc;
     for (uint32_t i = 0; i < n; i++) {
         ChunkDesc &d = s.h_desc[i];
         d.src = d_src + src_off[i];
         d.dst = d_dst + dst_off[i];
         d.len = src_len[i];
-        const uint64_t nb = (src_len[i] + kBlock - 1) / kBlock;
-        if (nb >= (1ull << 24)) return SKY_E_CAPACITY;
-        d.nblk = (uint32_t)nb;
-        d.group = 0;
-        rows = std::max(rows, d.nblk);
+        d.nblk = (uint32_t)nblocks(src_len[i]);
         s.h_chain[i] = 15;  // block 0 starts right after the 15-byte frame header
     }
-    if ((uint64_t)rows * n >= 0xffffffffull) return SKY_E_CAPACITY;
-    // MD5 lane assignment: longest chunks first so a warp's 32 lanes carry similar lengths
-    const uint32_t ng = (n + 31) / 32;
-    std::iota(s.h_order, s.h_order + n, 0u);
-    std::stable_sort(s.h_order, s.h_order + n, [&](uint32_t a, uint32_t b) { return src_len[a] > src_len[b]; });
-    for (uint32_t i = n; i < ng * 32; i++) s.h_order[i] = 0xffffffffu;
+    const uint32_t ng = md5_lane_order(s.h_order, n, src_len);
     for (uint32_t i = 0; i < n; i++) s.h_desc[s.h_order[i]].group = i / 32;
 
     CK(ctx, cudaMemcpyAsync(s.d_desc, s.h_desc, n * sizeof(ChunkDesc), cudaMemcpyHostToDevice, meta_st));
@@ -1070,10 +1084,8 @@ static int launch_batch(sky_ctx *ctx, Slot &s, cudaStream_t st, cudaStream_t met
     CK(ctx, cudaGetLastError());
     CK(ctx, cudaEventRecord(s.ev_k1, st));
     ctx->launches++;
-    if (flags & SKY_F_E2EE) {
-        int rc = launch_seal(ctx, s, st, n, d_dst, flags);
-        if (rc != SKY_OK) return rc;
-    }
+    if (flags & SKY_F_E2EE)
+        if (int rc = launch_seal(ctx, s, st, n, d_dst, flags)) return rc;
     CK(ctx, cudaEventRecord(s.ev_res, st));  // kernel(s) done => sizes + digests are in host memory
     return SKY_OK;
 }
@@ -1086,7 +1098,7 @@ static int issue_d2h(sky_ctx *ctx, Slot &s) {
     if (ctx->trace) CK(ctx, cudaEventRecord(s.ev_d0, ctx->st_d2h));
     for (uint32_t i = 0; i < s.n; i++) {
         if (s.h_outlen[i] == 0) continue;  // MD5-only batch without E2EE: nothing comes back but the digests
-        const uint8_t *from = (s.flags & SKY_F_E2EE) ? s.d_box + s.out_off[i] + 64ull * i + 8 : s.d_out + s.out_off[i];
+        const uint8_t *from = (s.flags & SKY_F_E2EE) ? s.d_box + box_offset(s.out_off[i], i) : s.d_out + s.out_off[i];
         CK(ctx, cudaMemcpyAsync(s.dst[i], from, s.h_outlen[i], cudaMemcpyDeviceToHost, ctx->st_d2h));
     }
     if (ctx->trace) CK(ctx, cudaEventRecord(s.ev_d1, ctx->st_d2h));
@@ -1100,8 +1112,7 @@ static int progress(sky_ctx *ctx) {
         cudaError_t q = cudaEventQuery(s.ev_res);
         if (q == cudaErrorNotReady) continue;
         CK(ctx, q);
-        int rc = issue_d2h(ctx, s);
-        if (rc != SKY_OK) return rc;
+        if (int rc = issue_d2h(ctx, s)) return rc;
     }
     return SKY_OK;
 }
@@ -1109,21 +1120,22 @@ static int progress(sky_ctx *ctx) {
 int sky_process_device(sky_ctx *ctx, uint32_t n, const void *d_src, const uint64_t *src_off, const uint64_t *src_len,
                        void *d_dst, const uint64_t *dst_off, const uint64_t *dst_cap, uint32_t flags, void *stream,
                        uint64_t *out_len, uint8_t *md5, float *kernel_ms) {
-    if (!ctx || n == 0 || !src_off || !src_len || !dst_off || !dst_cap || !d_dst) return SKY_E_INVALID;
-    if (flags & SKY_F_E2EE) return SKY_E_INVALID;  // boxes are a host-path feature (sky_submit_flags)
-    if (n > ctx->max_chunks) return SKY_E_CAPACITY;
-    if ((reinterpret_cast<uintptr_t>(d_src) & 15) || (reinterpret_cast<uintptr_t>(d_dst) & 15)) return SKY_E_INVALID;
+    if (!ctx || n == 0 || !src_off || !src_len || !dst_off || !dst_cap || !d_dst) return fail(ctx, SKY_E_INVALID, "NULL argument or n == 0");
+    if (flags & SKY_F_E2EE) return fail(ctx, SKY_E_INVALID, "SKY_F_E2EE is a host-path feature (sky_submit_flags)");
+    if (n > ctx->max_chunks) return fail(ctx, SKY_E_CAPACITY, "n = %u > max_chunks = %u", n, ctx->max_chunks);
+    if ((reinterpret_cast<uintptr_t>(d_src) & 15) || (reinterpret_cast<uintptr_t>(d_dst) & 15))
+        return fail(ctx, SKY_E_INVALID, "d_src or d_dst is not 16-byte aligned");
     for (uint32_t i = 0; i < n; i++) {
-        if ((src_off[i] & 15) || (dst_off[i] & 15)) return SKY_E_INVALID;
-        if (dst_cap[i] < sky_frame_bound(src_len[i])) return SKY_E_CAPACITY;
-        if (src_len[i] && !d_src) return SKY_E_INVALID;
+        if ((src_off[i] & 15) || (dst_off[i] & 15)) return fail(ctx, SKY_E_INVALID, "src_off[%u] or dst_off[%u] is not a multiple of 16", i, i);
+        if (dst_cap[i] < sky_frame_bound(src_len[i])) return fail(ctx, SKY_E_CAPACITY, "dst_cap[%u] < sky_frame_bound(src_len[%u])", i, i);
+        if (src_len[i] && !d_src) return fail(ctx, SKY_E_INVALID, "d_src is NULL");
     }
     CK(ctx, cudaSetDevice(ctx->device));
     Slot &s = ctx->slots[0];
-    if (s.busy) return SKY_E_BUSY;
+    if (s.busy) return fail(ctx, SKY_E_BUSY, "slot 0 holds a batch that was not waited for");
     cudaStream_t st = stream ? (cudaStream_t)stream : s.stream;
-    int rc = launch_batch(ctx, s, st, st, n, (const uint8_t *)d_src, src_off, src_len, (uint8_t *)d_dst, dst_off, flags);
-    if (rc != SKY_OK) return rc;
+    flags = with_default_stages(flags);
+    if (int rc = launch_batch(ctx, s, st, st, n, (const uint8_t *)d_src, src_off, src_len, (uint8_t *)d_dst, dst_off, flags)) return rc;
     CK(ctx, cudaStreamSynchronize(st));
     if (out_len) memcpy(out_len, s.h_outlen, n * sizeof(uint64_t));
     if (md5) memcpy(md5, s.h_md5, (size_t)n * 16);
@@ -1138,34 +1150,31 @@ int sky_submit(sky_ctx *ctx, uint32_t n, const void *const *src, const uint64_t 
 
 int sky_submit_flags(sky_ctx *ctx, uint32_t n, const void *const *src, const uint64_t *src_len, void *const *dst,
                      const uint64_t *dst_cap, uint32_t flags, const uint8_t *nonces, uint64_t *ticket) {
-    if (!ctx || n == 0 || !src || !src_len || !ticket) return SKY_E_INVALID;
-    if ((flags & (SKY_F_LZ4 | SKY_F_MD5)) == 0) flags |= SKY_F_LZ4 | SKY_F_MD5;
+    if (!ctx || n == 0 || !src || !src_len || !ticket) return fail(ctx, SKY_E_INVALID, "NULL argument or n == 0");
+    flags = with_default_stages(flags);
     const bool e2ee = (flags & SKY_F_E2EE) != 0, frames = (flags & SKY_F_LZ4) != 0;
     const bool returns_data = frames || e2ee;  // MD5-only without E2EE: only digests come back
-    if (returns_data && (!dst || !dst_cap)) return SKY_E_INVALID;
-    if (e2ee && (!ctx->d_key || !nonces)) return SKY_E_NOKEY;
-    if (n > ctx->max_chunks) return SKY_E_CAPACITY;
+    if (returns_data && (!dst || !dst_cap)) return fail(ctx, SKY_E_INVALID, "dst or dst_cap is NULL");
+    if (e2ee && (!ctx->d_key || !nonces)) return fail(ctx, SKY_E_NOKEY, ctx->d_key ? "nonces is NULL" : "no key (sky_set_e2ee_key)");
+    if (n > ctx->max_chunks) return fail(ctx, SKY_E_CAPACITY, "n = %u > max_chunks = %u", n, ctx->max_chunks);
     Slot *sp = nullptr;
     for (auto &s : ctx->slots)
         if (!s.busy && s.d_in) { sp = &s; break; }
-    if (!sp) return ctx->slots[0].d_in ? SKY_E_BUSY : SKY_E_INVALID;
+    if (!sp)
+        return ctx->slots[0].d_in ? fail(ctx, SKY_E_BUSY, "all %zu slots hold batches that were not waited for", ctx->slots.size())
+                                  : fail(ctx, SKY_E_INVALID, "the ctx was created without slots (n_slots = 0)");
     Slot &s = *sp;
     CK(ctx, cudaSetDevice(ctx->device));
-    { int prc = progress(ctx); if (prc != SKY_OK) return prc; }
-    std::vector<uint64_t> in_off(n), out_off(n);
-    uint64_t ip = 0, op = 0;
+    if (int rc = progress(ctx)) return rc;
     for (uint32_t i = 0; i < n; i++) {
-        if (src_len[i] && !src[i]) return SKY_E_INVALID;
-        if (returns_data) {
-            const uint64_t need = (frames ? sky_frame_bound(src_len[i]) : src_len[i]) + (e2ee ? kBoxOverhead : 0);
-            if (!dst[i] || dst_cap[i] < need) return SKY_E_CAPACITY;
-        }
-        in_off[i] = ip;
-        out_off[i] = op;
-        ip += round16(src_len[i]);
-        op += round16(sky_frame_bound(src_len[i]));
+        if (src_len[i] && !src[i]) return fail(ctx, SKY_E_INVALID, "src[%u] is NULL", i);
+        const uint64_t need = (frames ? sky_frame_bound(src_len[i]) : src_len[i]) + (e2ee ? kBoxOverhead : 0);
+        if (returns_data && (!dst[i] || dst_cap[i] < need)) return fail(ctx, SKY_E_CAPACITY, "dst[%u] is NULL or dst_cap[%u] < %" PRIu64, i, i, need);
     }
-    if (ip > ctx->in_cap || op > ctx->out_cap) return SKY_E_CAPACITY;
+    uint64_t in_end, out_end;
+    std::vector<uint64_t> in_off = pack16(n, [&](uint32_t i) { return src_len[i]; }, in_end);
+    std::vector<uint64_t> out_off = pack16(n, [&](uint32_t i) { return sky_frame_bound(src_len[i]); }, out_end);
+    if (in_end > ctx->in_cap || out_end > ctx->out_cap) return fail(ctx, SKY_E_CAPACITY, "the batch exceeds a slot's input or frame slab");
     if (ctx->trace) CK(ctx, cudaEventRecord(s.ev_h0, ctx->st_h2d));
     for (uint32_t i = 0; i < n; i++)
         if (src_len[i]) CK(ctx, cudaMemcpyAsync(s.d_in + in_off[i], src[i], src_len[i], cudaMemcpyHostToDevice, ctx->st_h2d));
@@ -1178,8 +1187,8 @@ int sky_submit_flags(sky_ctx *ctx, uint32_t n, const void *const *src, const uin
         CK(ctx, cudaMemcpyAsync(s.d_nonce, s.h_nonce, 24ull * n, cudaMemcpyHostToDevice, ctx->st_h2d));
     }
     s.flags = flags;
-    int rc = launch_batch(ctx, s, s.stream, ctx->st_h2d, n, s.d_in, in_off.data(), src_len, s.d_out, out_off.data(), flags | SKY_F_NO_PACING);
-    if (rc != SKY_OK) return rc;
+    if (int rc = launch_batch(ctx, s, s.stream, ctx->st_h2d, n, s.d_in, in_off.data(), src_len, s.d_out, out_off.data(), flags | SKY_F_NO_PACING))
+        return rc;
     s.busy = true;
     s.d2h_issued = false;
     s.ticket = ctx->next_ticket++;
@@ -1191,20 +1200,19 @@ int sky_submit_flags(sky_ctx *ctx, uint32_t n, const void *const *src, const uin
 }
 
 int sky_wait(sky_ctx *ctx, uint64_t ticket, uint64_t *out_len, uint8_t *md5, float *kernel_ms) {
-    if (!ctx) return SKY_E_INVALID;
+    if (!ctx) return fail(ctx, SKY_E_INVALID, "ctx is NULL");
     Slot *sp = nullptr;
     for (auto &s : ctx->slots)
         if (s.busy && s.ticket == ticket) { sp = &s; break; }
-    if (!sp) return SKY_E_TICKET;
+    if (!sp) return fail(ctx, SKY_E_TICKET, "ticket %" PRIu64 " is not in flight", ticket);
     Slot &s = *sp;
     CK(ctx, cudaSetDevice(ctx->device));
-    { int prc = progress(ctx); if (prc != SKY_OK) return prc; }
+    if (int rc = progress(ctx)) return rc;
     if (!s.d2h_issued) {
         CK(ctx, cudaEventSynchronize(s.ev_res));  // sizes + digests are on the host now
-        int rc = issue_d2h(ctx, s);
-        if (rc != SKY_OK) return rc;
+        if (int rc = issue_d2h(ctx, s)) return rc;
     }
-    { int prc = progress(ctx); if (prc != SKY_OK) return prc; }  // let later batches' copies queue up behind ours
+    if (int rc = progress(ctx)) return rc;  // let later batches' copies queue up behind ours
     CK(ctx, cudaEventSynchronize(s.ev_d2h));
     if (out_len) memcpy(out_len, s.h_outlen, s.n * sizeof(uint64_t));
     if (md5) memcpy(md5, s.h_md5, (size_t)s.n * 16);
@@ -1225,89 +1233,77 @@ int sky_wait(sky_ctx *ctx, uint64_t ticket, uint64_t *out_len, uint8_t *md5, flo
 }
 
 int sky_device_alloc(sky_ctx *ctx, uint64_t bytes, void **dptr) {
-    if (!ctx || !dptr) return SKY_E_INVALID;
+    if (!ctx || !dptr) return fail(ctx, SKY_E_INVALID, "ctx or dptr is NULL");
     CK(ctx, cudaSetDevice(ctx->device));
-    cudaError_t e = cudaMalloc(dptr, bytes ? bytes : 16);
-    if (e != cudaSuccess) { ctx->err = cudaGetErrorString(e); return SKY_E_NOMEM; }
+    const cudaError_t e = cudaMalloc(dptr, bytes ? bytes : 16);
+    if (e != cudaSuccess) return fail(ctx, SKY_E_NOMEM, "cudaMalloc(%" PRIu64 ") -> %s", bytes, cudaGetErrorString(e));
     return SKY_OK;
 }
 int sky_device_free(sky_ctx *ctx, void *dptr) {
-    if (!ctx) return SKY_E_INVALID;
+    if (!ctx) return fail(ctx, SKY_E_INVALID, "ctx is NULL");
     CK(ctx, cudaSetDevice(ctx->device));
     CK(ctx, cudaFree(dptr));
     return SKY_OK;
 }
 int sky_memcpy_h2d(sky_ctx *ctx, void *dptr, const void *host, uint64_t bytes) {
-    if (!ctx) return SKY_E_INVALID;
+    if (!ctx) return fail(ctx, SKY_E_INVALID, "ctx is NULL");
     CK(ctx, cudaSetDevice(ctx->device));
     CK(ctx, cudaMemcpy(dptr, host, bytes, cudaMemcpyHostToDevice));
     return SKY_OK;
 }
 int sky_memcpy_d2h(sky_ctx *ctx, void *host, const void *dptr, uint64_t bytes) {
-    if (!ctx) return SKY_E_INVALID;
+    if (!ctx) return fail(ctx, SKY_E_INVALID, "ctx is NULL");
     CK(ctx, cudaSetDevice(ctx->device));
     CK(ctx, cudaMemcpy(host, dptr, bytes, cudaMemcpyDeviceToHost));
     return SKY_OK;
 }
 
-
 // ---------------------------------------------------------------------------------- receiver side
 // Enqueues index + decode (+ MD5 of the decoded bytes through the fused kernel's MD5 role) on `st`.
 static int launch_decode(sky_ctx *ctx, Slot &s, cudaStream_t st, uint32_t n, const uint8_t *d_frames, const uint64_t *frame_off,
                          const uint64_t *frame_len, uint8_t *d_out, const uint64_t *out_off, const uint64_t *raw_len) {
+    uint32_t rows;
+    if (int rc = block_rows(ctx, n, raw_len, &rows)) return rc;
     uint64_t nblk_total = 0;
-    uint32_t rows = 1;
     for (uint32_t i = 0; i < n; i++) {
         DecChunk &d = s.h_dchunks[i];
         d.frame = d_frames + frame_off[i];
         d.out = d_out + out_off[i];
         d.frame_len = frame_len[i];
         d.raw_len = raw_len[i];
-        const uint64_t nb = (raw_len[i] + kBlock - 1) / kBlock;
-        if (nb >= (1ull << 24)) return SKY_E_CAPACITY;
-        d.nblk = (uint32_t)nb;
+        d.nblk = (uint32_t)nblocks(raw_len[i]);
         d.blk_base = nblk_total;
         d.linked = 0;
-        nblk_total += nb;
-        rows = std::max(rows, d.nblk);
+        nblk_total += d.nblk;
     }
-    if ((uint64_t)rows * n >= 0xffffffffull) return SKY_E_CAPACITY;
-    if (nblk_total + 1 > s.dblocks_cap) {
+    if (nblk_total + 1 > s.dblocks_cap) {  // grow the block arrays (the previous decode on `st` may still use them)
         CK(ctx, cudaStreamSynchronize(st));
-        cudaFree(s.d_dblocks);
-        cudaFree(s.d_blkdone);
-        s.d_dblocks = nullptr;
-        s.d_blkdone = nullptr;
         s.dblocks_cap = 0;
-        CK(ctx, cudaMalloc(&s.d_dblocks, (nblk_total + 1) * sizeof(DecBlock)));
-        CK(ctx, cudaMalloc(&s.d_blkdone, (nblk_total + 1) * sizeof(uint32_t)));
+        CK(ctx, cudaMalloc(s.d_dblocks.put(), (nblk_total + 1) * sizeof(DecBlock)));
+        CK(ctx, cudaMalloc(s.d_block_flags.put(), (nblk_total + 1) * sizeof(uint32_t)));
         s.dblocks_cap = nblk_total + 1;
     }
     CK(ctx, cudaMemcpyAsync(s.d_dchunks, s.h_dchunks, n * sizeof(DecChunk), cudaMemcpyHostToDevice, st));
     CK(ctx, cudaMemsetAsync(s.d_counters, 0, 64, st));
-    CK(ctx, cudaMemsetAsync(s.d_freed, 0, n * sizeof(uint32_t), st));
+    CK(ctx, cudaMemsetAsync(s.d_blocks_done, 0, n * sizeof(uint32_t), st));
     CK(ctx, cudaMemsetAsync(s.d_dstatus, 0, n * sizeof(int32_t), st));
-    CK(ctx, cudaMemsetAsync(s.d_blkdone, 0, (nblk_total + 1) * sizeof(uint32_t), st));
-    // MD5 lane assignment: longest chunks first (same rule as the sender side)
-    const uint32_t ng = (n + 31) / 32;
-    std::iota(s.h_order, s.h_order + n, 0u);
-    std::stable_sort(s.h_order, s.h_order + n, [&](uint32_t a, uint32_t b) { return raw_len[a] > raw_len[b]; });
-    for (uint32_t i = n; i < ng * 32; i++) s.h_order[i] = 0xffffffffu;
+    CK(ctx, cudaMemsetAsync(s.d_block_flags, 0, (nblk_total + 1) * sizeof(uint32_t), st));
+    const uint32_t ng = md5_lane_order(s.h_order, n, raw_len);
     CK(ctx, cudaMemcpyAsync(s.d_order, s.h_order, ng * 32 * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
     memset(s.h_md5, 0, (size_t)n * 16);
     DecParams p;
     p.chunks = s.d_dchunks;
     p.blocks = s.d_dblocks;
     p.status = s.d_dstatus;
-    p.done = s.d_freed;
+    p.done = s.d_blocks_done;
     p.counter = s.d_counters;
-    p.blk_done = s.d_blkdone;
+    p.blk_done = s.d_block_flags;
     p.md5_order = s.d_order;
     p.md5_out = s.d_md5;
     p.n_chunks = n;
     p.n_groups = ng;
     p.rows = rows;
-    CK(ctx, cudaEventRecord(s.ev_h0, st));  // start marker of the receiver-side kernels
+    CK(ctx, cudaEventRecord(s.ev_k0, st));
     sky_frame_index_kernel<<<(n + 127) / 128, 128, 0, st>>>(p);
     CK(ctx, cudaGetLastError());
     sky_decode_kernel<<<ctx->sm_count, 512, kMd5WarpsPerCta * kRingBytes, st>>>(p);
@@ -1321,23 +1317,22 @@ static int launch_decode(sky_ctx *ctx, Slot &s, cudaStream_t st, uint32_t n, con
 int sky_decode_device(sky_ctx *ctx, uint32_t n, const void *d_frames, const uint64_t *frame_off, const uint64_t *frame_len,
                       void *d_out, const uint64_t *out_off, const uint64_t *raw_len, void *stream, int32_t *status, uint8_t *md5,
                       float *kernel_ms) {
-    if (!ctx || n == 0 || !d_frames || !frame_off || !frame_len || !out_off || !raw_len) return SKY_E_INVALID;
-    if (n > ctx->max_chunks) return SKY_E_CAPACITY;
-    if (reinterpret_cast<uintptr_t>(d_out) & 15) return SKY_E_INVALID;
+    if (!ctx || n == 0 || !d_frames || !frame_off || !frame_len || !out_off || !raw_len) return fail(ctx, SKY_E_INVALID, "NULL argument or n == 0");
+    if (n > ctx->max_chunks) return fail(ctx, SKY_E_CAPACITY, "n = %u > max_chunks = %u", n, ctx->max_chunks);
+    if (reinterpret_cast<uintptr_t>(d_out) & 15) return fail(ctx, SKY_E_INVALID, "d_out is not 16-byte aligned");
     for (uint32_t i = 0; i < n; i++) {
-        if (out_off[i] & 15) return SKY_E_INVALID;
-        if (raw_len[i] && !d_out) return SKY_E_INVALID;
+        if (out_off[i] & 15) return fail(ctx, SKY_E_INVALID, "out_off[%u] is not a multiple of 16", i);
+        if (raw_len[i] && !d_out) return fail(ctx, SKY_E_INVALID, "d_out is NULL");
     }
     CK(ctx, cudaSetDevice(ctx->device));
     Slot &s = ctx->slots[0];
-    if (s.busy) return SKY_E_BUSY;
+    if (s.busy) return fail(ctx, SKY_E_BUSY, "slot 0 holds a batch that was not waited for");
     cudaStream_t st = stream ? (cudaStream_t)stream : s.stream;
-    int rc = launch_decode(ctx, s, st, n, (const uint8_t *)d_frames, frame_off, frame_len, (uint8_t *)d_out, out_off, raw_len);
-    if (rc != SKY_OK) return rc;
+    if (int rc = launch_decode(ctx, s, st, n, (const uint8_t *)d_frames, frame_off, frame_len, (uint8_t *)d_out, out_off, raw_len)) return rc;
     CK(ctx, cudaStreamSynchronize(st));
     if (status) memcpy(status, s.h_dstatus, n * sizeof(int32_t));
     if (md5) memcpy(md5, s.h_md5, (size_t)n * 16);
-    if (kernel_ms) CK(ctx, cudaEventElapsedTime(kernel_ms, s.ev_h0, s.ev_k1));  // index + decode + MD5
+    if (kernel_ms) CK(ctx, cudaEventElapsedTime(kernel_ms, s.ev_k0, s.ev_k1));  // index + decode + MD5
     return SKY_OK;
 }
 
@@ -1348,38 +1343,33 @@ int sky_decode(sky_ctx *ctx, uint32_t n, const void *const *frames, const uint64
 
 int sky_decode_flags(sky_ctx *ctx, uint32_t n, const void *const *frames, const uint64_t *frame_len, void *const *dst,
                      const uint64_t *raw_len, uint32_t flags, int32_t *status, uint8_t *md5, float *kernel_ms) {
-    if (!ctx || n == 0 || !frames || !frame_len || !dst || !raw_len) return SKY_E_INVALID;
-    if (n > ctx->max_chunks) return SKY_E_CAPACITY;
+    if (!ctx || n == 0 || !frames || !frame_len || !dst || !raw_len) return fail(ctx, SKY_E_INVALID, "NULL argument or n == 0");
+    if (n > ctx->max_chunks) return fail(ctx, SKY_E_CAPACITY, "n = %u > max_chunks = %u", n, ctx->max_chunks);
     Slot &s = ctx->slots[0];
-    if (s.busy) return SKY_E_BUSY;
-    if (!s.d_in) return SKY_E_INVALID;  // ctx created without slabs
+    if (s.busy) return fail(ctx, SKY_E_BUSY, "slot 0 holds a batch that was not waited for");
+    if (!s.d_in) return fail(ctx, SKY_E_INVALID, "the ctx was created without slots (n_slots = 0)");
     const bool e2ee = (flags & SKY_F_E2EE) != 0;
-    if (e2ee && !ctx->d_key) return SKY_E_NOKEY;
+    if (e2ee && !ctx->d_key) return fail(ctx, SKY_E_NOKEY, "no key (sky_set_e2ee_key)");
     CK(ctx, cudaSetDevice(ctx->device));
+    for (uint32_t i = 0; i < n; i++)
+        if (!frames[i] || (raw_len[i] && !dst[i])) return fail(ctx, SKY_E_INVALID, "frames[%u] or dst[%u] is NULL", i, i);
     // roles swap on the way back: frames (<= bound) go into the frame slab, decoded bytes into the input slab
-    std::vector<uint64_t> f_off(n), o_off(n), f_len(frame_len, frame_len + n);
-    uint64_t fp = 0, op = 0;
-    for (uint32_t i = 0; i < n; i++) {
-        if (!frames[i] || (raw_len[i] && !dst[i])) return SKY_E_INVALID;
-        f_off[i] = fp;
-        o_off[i] = op;
-        fp += round16(frame_len[i]);
-        op += round16(raw_len[i]);
-    }
-    if (fp > ctx->out_cap || op > ctx->in_cap) return SKY_E_CAPACITY;
+    uint64_t f_end, o_end;
+    const std::vector<uint64_t> f_off = pack16(n, [&](uint32_t i) { return frame_len[i]; }, f_end);
+    const std::vector<uint64_t> o_off = pack16(n, [&](uint32_t i) { return raw_len[i]; }, o_end);
+    if (f_end > ctx->out_cap || o_end > ctx->in_cap) return fail(ctx, SKY_E_CAPACITY, "the batch exceeds slot 0's frame or output slab");
+    std::vector<uint64_t> f_len(frame_len, frame_len + n);
     if (e2ee) {
         // the payloads are boxes (nonce | tag | ciphertext): check the tags, decrypt into the frame slab, then decode as usual
-        int rc = alloc_box(ctx, s);
-        if (rc != SKY_OK) return rc;
+        if (int rc = alloc_box(ctx, s)) return rc;
         for (uint32_t i = 0; i < n; i++) {
-            s.h_boxmeta[i] = f_off[i] + 64ull * i;
-            s.h_boxmeta[n + i] = frame_len[i];
-            s.h_boxmeta[2 * n + i] = f_off[i];
-            CK(ctx, cudaMemcpyAsync(s.d_box + f_off[i] + 64ull * i + 8, frames[i], frame_len[i], cudaMemcpyHostToDevice, s.stream));
+            s.h_boxmeta[i] = frame_len[i];
+            s.h_boxmeta[n + i] = f_off[i];
+            CK(ctx, cudaMemcpyAsync(s.d_box + box_offset(f_off[i], i), frames[i], frame_len[i], cudaMemcpyHostToDevice, s.stream));
             f_len[i] = frame_len[i] >= (uint64_t)kBoxOverhead ? frame_len[i] - kBoxOverhead : 0;
         }
-        CK(ctx, cudaMemcpyAsync(s.d_boxmeta, s.h_boxmeta, 3ull * n * sizeof(uint64_t), cudaMemcpyHostToDevice, s.stream));
-        sky_box_open_setup_kernel<<<1, 256, 0, s.stream>>>(s.d_bchunks, s.d_blkbase, n, s.d_boxmeta, s.d_boxmeta + n, s.d_boxmeta + 2 * n, s.d_out, s.d_box);
+        CK(ctx, cudaMemcpyAsync(s.d_boxmeta, s.h_boxmeta, 2ull * n * sizeof(uint64_t), cudaMemcpyHostToDevice, s.stream));
+        sky_box_open_setup_kernel<<<1, 256, 0, s.stream>>>(s.d_bchunks, s.d_blkbase, n, s.d_boxmeta, s.d_boxmeta + n, s.d_out, s.d_box);
         CK(ctx, cudaGetLastError());
         sky_box_keys_kernel<<<(n + 63) / 64, 64, 0, s.stream>>>(s.d_bchunks, n, ctx->d_key, s.d_sub);
         CK(ctx, cudaGetLastError());
@@ -1393,8 +1383,8 @@ int sky_decode_flags(sky_ctx *ctx, uint32_t n, const void *const *frames, const 
         for (uint32_t i = 0; i < n; i++)
             CK(ctx, cudaMemcpyAsync(s.d_out + f_off[i], frames[i], frame_len[i], cudaMemcpyHostToDevice, s.stream));
     }
-    int rc = sky_decode_device(ctx, n, s.d_out, f_off.data(), f_len.data(), s.d_in, o_off.data(), raw_len, s.stream, status, md5, kernel_ms);
-    if (rc != SKY_OK) return rc;
+    if (int rc = sky_decode_device(ctx, n, s.d_out, f_off.data(), f_len.data(), s.d_in, o_off.data(), raw_len, s.stream, status, md5, kernel_ms))
+        return rc;
     if (e2ee) {
         for (uint32_t i = 0; i < n; i++)
             if (s.h_bstatus[i] != 0 || frame_len[i] < (uint64_t)kBoxOverhead) {  // forged or truncated box: never hand its bytes out

@@ -21,14 +21,37 @@ D_OK, D_BAD_HEADER, D_CORRUPT, D_SIZE, D_UNSUPPORTED, D_LAYOUT, D_TRUNCATED, D_A
 D_NAMES = {0: "ok", -1: "bad frame header", -2: "corrupt block", -3: "size mismatch", -4: "unsupported frame feature",
            -5: "unexpected block layout", -6: "truncated frame", -7: "box authentication failed"}
 
-# every symbol include/skychunk.h declares (tests check the .so exports exactly these)
-ABI_SYMBOLS = (
-    "sky_strerror", "sky_last_error", "sky_abi_version", "sky_device_count", "sky_device_pci_bus_id", "sky_kernel_config", "sky_frame_bound",
-    "sky_ctx_create", "sky_ctx_destroy", "sky_pinned_alloc", "sky_pinned_free",
-    "sky_submit", "sky_wait", "sky_submit_flags", "sky_set_e2ee_key", "sky_box_bound", "sky_process_device", "sky_decode_device", "sky_decode",
-    "sky_decode_flags",
-    "sky_device_alloc", "sky_device_free", "sky_memcpy_h2d", "sky_memcpy_d2h", "sky_launch_count",
-)
+_vp, _u64, _u32, _i32, _str = ctypes.c_void_p, ctypes.c_uint64, ctypes.c_uint32, ctypes.c_int, ctypes.c_char_p
+_p_vp, _p_u64, _p_i32, _p_f32 = (ctypes.POINTER(t) for t in (_vp, _u64, _i32, ctypes.c_float))
+# every symbol include/skychunk.h declares, name: (restype, argtypes) (tests check the .so exports exactly these)
+_ABI = {
+    "sky_strerror": (_str, [_i32]),
+    "sky_last_error": (_str, [_vp]),
+    "sky_abi_version": (_i32, []),
+    "sky_device_count": (_i32, [_p_i32]),
+    "sky_device_pci_bus_id": (_i32, [_i32, _str, _i32]),
+    "sky_kernel_config": (_u32, [_i32]),
+    "sky_frame_bound": (_u64, [_u64]),
+    "sky_ctx_create": (_i32, [_i32, _u64, _u32, _u32, _p_vp]),
+    "sky_ctx_destroy": (_i32, [_vp]),
+    "sky_pinned_alloc": (_vp, [_u64]),
+    "sky_pinned_free": (_i32, [_vp]),
+    "sky_submit": (_i32, [_vp, _u32, _p_vp, _p_u64, _p_vp, _p_u64, _p_u64]),
+    "sky_wait": (_i32, [_vp, _u64, _p_u64, _vp, _p_f32]),
+    "sky_submit_flags": (_i32, [_vp, _u32, _p_vp, _p_u64, _p_vp, _p_u64, _u32, _str, _p_u64]),
+    "sky_set_e2ee_key": (_i32, [_vp, _str]),
+    "sky_box_bound": (_u64, [_u64]),
+    "sky_process_device": (_i32, [_vp, _u32, _vp, _p_u64, _p_u64, _vp, _p_u64, _p_u64, _u32, _vp, _p_u64, _vp, _p_f32]),
+    "sky_decode_device": (_i32, [_vp, _u32, _vp, _p_u64, _p_u64, _vp, _p_u64, _p_u64, _vp, _p_i32, _vp, _p_f32]),
+    "sky_decode": (_i32, [_vp, _u32, _p_vp, _p_u64, _p_vp, _p_u64, _p_i32, _vp, _p_f32]),
+    "sky_decode_flags": (_i32, [_vp, _u32, _p_vp, _p_u64, _p_vp, _p_u64, _u32, _p_i32, _vp, _p_f32]),
+    "sky_device_alloc": (_i32, [_vp, _u64, _p_vp]),
+    "sky_device_free": (_i32, [_vp, _vp]),
+    "sky_memcpy_h2d": (_i32, [_vp, _vp, _vp, _u64]),
+    "sky_memcpy_d2h": (_i32, [_vp, _vp, _vp, _u64]),
+    "sky_launch_count": (_u64, [_vp]),
+}
+ABI_SYMBOLS = tuple(_ABI)
 
 
 class SkyChunkError(RuntimeError):
@@ -66,59 +89,9 @@ def lib() -> ctypes.CDLL:
         if _build.needs_build():
             _build.build()
         L = ctypes.CDLL(str(LIB_PATH))
-    vp, u64, u32, i32 = ctypes.c_void_p, ctypes.c_uint64, ctypes.c_uint32, ctypes.c_int
-    p_u64 = ctypes.POINTER(u64)
-    L.sky_strerror.argtypes = [i32]
-    L.sky_strerror.restype = ctypes.c_char_p
-    L.sky_last_error.argtypes = [vp]
-    L.sky_last_error.restype = ctypes.c_char_p
-    L.sky_abi_version.argtypes = []
-    L.sky_abi_version.restype = i32
-    L.sky_device_count.argtypes = [ctypes.POINTER(i32)]
-    L.sky_device_count.restype = i32
-    L.sky_device_pci_bus_id.argtypes = [i32, ctypes.c_char_p, i32]
-    L.sky_device_pci_bus_id.restype = i32
-    L.sky_kernel_config.argtypes = [i32]
-    L.sky_kernel_config.restype = u32
-    L.sky_frame_bound.argtypes = [u64]
-    L.sky_frame_bound.restype = u64
-    L.sky_ctx_create.argtypes = [i32, u64, u32, u32, ctypes.POINTER(vp)]
-    L.sky_ctx_create.restype = i32
-    L.sky_ctx_destroy.argtypes = [vp]
-    L.sky_ctx_destroy.restype = i32
-    L.sky_pinned_alloc.argtypes = [u64]
-    L.sky_pinned_alloc.restype = vp
-    L.sky_pinned_free.argtypes = [vp]
-    L.sky_pinned_free.restype = i32
-    L.sky_submit.argtypes = [vp, u32, ctypes.POINTER(vp), p_u64, ctypes.POINTER(vp), p_u64, p_u64]
-    L.sky_submit.restype = i32
-    L.sky_submit_flags.argtypes = [vp, u32, ctypes.POINTER(vp), p_u64, ctypes.POINTER(vp), p_u64, u32, ctypes.c_char_p, p_u64]
-    L.sky_submit_flags.restype = i32
-    L.sky_set_e2ee_key.argtypes = [vp, ctypes.c_char_p]
-    L.sky_set_e2ee_key.restype = i32
-    L.sky_box_bound.argtypes = [u64]
-    L.sky_box_bound.restype = u64
-    L.sky_wait.argtypes = [vp, u64, p_u64, vp, ctypes.POINTER(ctypes.c_float)]
-    L.sky_wait.restype = i32
-    L.sky_process_device.argtypes = [vp, u32, vp, p_u64, p_u64, vp, p_u64, p_u64, u32, vp, p_u64, vp, ctypes.POINTER(ctypes.c_float)]
-    L.sky_process_device.restype = i32
-    p_i32 = ctypes.POINTER(ctypes.c_int32)
-    L.sky_decode_device.argtypes = [vp, u32, vp, p_u64, p_u64, vp, p_u64, p_u64, vp, p_i32, vp, ctypes.POINTER(ctypes.c_float)]
-    L.sky_decode_device.restype = i32
-    L.sky_decode.argtypes = [vp, u32, ctypes.POINTER(vp), p_u64, ctypes.POINTER(vp), p_u64, p_i32, vp, ctypes.POINTER(ctypes.c_float)]
-    L.sky_decode.restype = i32
-    L.sky_decode_flags.argtypes = [vp, u32, ctypes.POINTER(vp), p_u64, ctypes.POINTER(vp), p_u64, u32, p_i32, vp, ctypes.POINTER(ctypes.c_float)]
-    L.sky_decode_flags.restype = i32
-    L.sky_device_alloc.argtypes = [vp, u64, ctypes.POINTER(vp)]
-    L.sky_device_alloc.restype = i32
-    L.sky_device_free.argtypes = [vp, vp]
-    L.sky_device_free.restype = i32
-    L.sky_memcpy_h2d.argtypes = [vp, vp, vp, u64]
-    L.sky_memcpy_h2d.restype = i32
-    L.sky_memcpy_d2h.argtypes = [vp, vp, vp, u64]
-    L.sky_memcpy_d2h.restype = i32
-    L.sky_launch_count.argtypes = [vp]
-    L.sky_launch_count.restype = u64
+    for name, (restype, argtypes) in _ABI.items():
+        fn = getattr(L, name)
+        fn.restype, fn.argtypes = restype, argtypes
     _lib = L
     return L
 
@@ -145,6 +118,12 @@ def frame_bound(n: int) -> int:
 
 def round16(x: int) -> int:
     return (x + 15) & ~15
+
+
+def _split_digests(buf, n: int) -> list:
+    """n 16-byte MD5 digests packed back to back in `buf` -> list of bytes."""
+    raw = bytes(buf)
+    return [raw[16 * i : 16 * i + 16] for i in range(n)]
 
 
 def device_count() -> int:
@@ -249,8 +228,7 @@ class Context:
         md5 = (ctypes.c_ubyte * (16 * n))()
         ms = ctypes.c_float(0)
         self._check(lib().sky_wait(self._h, ticket, out, md5, ctypes.byref(ms)))
-        raw = bytes(md5)
-        return list(out), [raw[16 * i : 16 * i + 16] for i in range(n)], ms.value
+        return list(out), _split_digests(md5, n), ms.value
 
     # ------------------------------------------------------------------ device-resident path
     def process_device(self, d_src: int, src_off: Sequence[int], src_len: Sequence[int], d_dst: int, dst_off: Sequence[int],
@@ -265,8 +243,7 @@ class Context:
             lib().sky_process_device(self._h, n, d_src, U(*src_off), U(*src_len), d_dst, U(*dst_off), U(*dst_cap), flags,
                                      stream or None, out, md5, ctypes.byref(ms))
         )
-        raw = bytes(md5)
-        return list(out), [raw[16 * i : 16 * i + 16] for i in range(n)], ms.value
+        return list(out), _split_digests(md5, n), ms.value
 
     # ------------------------------------------------------------------ receiver side
     def decode_device(self, d_frames: int, frame_off: Sequence[int], frame_len: Sequence[int], d_out: int, out_off: Sequence[int],
@@ -279,8 +256,7 @@ class Context:
         ms = ctypes.c_float(0)
         self._check(lib().sky_decode_device(self._h, n, d_frames, U(*frame_off), U(*frame_len), d_out, U(*out_off), U(*raw_len),
                                             stream or None, st, md5, ctypes.byref(ms)))
-        raw = bytes(md5)
-        return list(st), [raw[16 * i : 16 * i + 16] for i in range(n)], ms.value
+        return list(st), _split_digests(md5, n), ms.value
 
     def decode(self, frame_addrs: Sequence[int], frame_lens: Sequence[int], dst_addrs: Sequence[int], raw_lens: Sequence[int], flags: int = 0):
         """Host buffers, synchronous. -> (status, digests, kernel_ms).  flags = F_E2EE: the payloads are sealed boxes."""
@@ -291,8 +267,7 @@ class Context:
         md5 = (ctypes.c_ubyte * (16 * n))()
         ms = ctypes.c_float(0)
         self._check(lib().sky_decode_flags(self._h, n, A(*frame_addrs), U(*frame_lens), A(*dst_addrs), U(*raw_lens), flags, st, md5, ctypes.byref(ms)))
-        raw = bytes(md5)
-        return list(st), [raw[16 * i : 16 * i + 16] for i in range(n)], ms.value
+        return list(st), _split_digests(md5, n), ms.value
 
     # ------------------------------------------------------------------ torch-free device memory
     def device_alloc(self, nbytes: int) -> int:

@@ -246,18 +246,24 @@ def test_stage_flags(ctx):
 # ---------------------------------------------------------------- ABI error behaviour
 def test_abi_argument_errors(ctx):
     d = ctx.device_alloc(4096)
+    misaligned = (([8], [10], [0], [64]), native.SKY_E_INVALID, "src_off[0] or dst_off[0] is not a multiple of 16")
+    too_small = (([0], [100], [0], [100]), native.SKY_E_CAPACITY, "dst_cap[0] < sky_frame_bound(src_len[0])")
     try:
-        with pytest.raises(native.SkyChunkError) as e:
-            ctx.process_device(d, [8], [10], d + 1024, [0], [64])  # misaligned src offset
-        assert e.value.code == native.SKY_E_INVALID
-        with pytest.raises(native.SkyChunkError) as e:
-            ctx.process_device(d, [0], [100], d + 1024, [0], [100])  # dst_cap < bound
-        assert e.value.code == native.SKY_E_CAPACITY
+        # invalid, capacity, invalid again on one ctx: each error's detail names its own cause, never an earlier one's
+        for (src_off, src_len, dst_off, dst_cap), code, cause in (misaligned, too_small, misaligned):
+            with pytest.raises(native.SkyChunkError) as e:
+                ctx.process_device(d, src_off, src_len, d + 1024, dst_off, dst_cap)
+            assert e.value.code == code
+            assert cause in str(e.value)
+            assert all(other not in str(e.value) for _, _, other in (misaligned, too_small) if other != cause)
         small = native.Context(0, 1 << 20, 2, 0)
         with pytest.raises(native.SkyChunkError) as e:
             small.process_device(d, [0, 16, 32], [1, 1, 1], d + 1024, [0, 32, 64], [32, 32, 32])
-        assert e.value.code == native.SKY_E_CAPACITY
+        assert e.value.code == native.SKY_E_CAPACITY and "n = 3 > max_chunks = 2" in str(e.value)
         small.close()
+        with pytest.raises(native.SkyChunkError) as e:  # no ctx to hold the detail: it is the calling thread's
+            native.Context(0, 1 << 20, 0, 0)
+        assert e.value.code == native.SKY_E_INVALID and "max_chunks == 0" in str(e.value)
     finally:
         ctx.device_free(d)
 

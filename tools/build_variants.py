@@ -11,8 +11,6 @@ VARIANTS = {
     "pa10_r3": {"SKY_PARSERS": 10, "SKY_RING_EXTRA": 3},
     "pa12_r2": {"SKY_PARSERS": 12, "SKY_RING_EXTRA": 2},  # the default build
     "pa13_r1": {"SKY_PARSERS": 13, "SKY_RING_EXTRA": 1},
-    "wait1024": {"SKY_WAIT_NS": 1024},
-    "pace1": {"SKY_PACE_LEAD": 1},
 }
 
 if __name__ == "__main__":
