@@ -17,7 +17,7 @@
  * Output format: one LZ4 frame per chunk that lz4.frame.decompress (gateway_receiver.py:196)
  * restores bit-exactly: magic, FLG=0x68 (v01, independent blocks, content size), BD=0x40 (64 KiB),
  * u64le content size, header checksum, blocks (bit 31 set = stored raw), EndMark.  A zero-length
- * chunk yields the 11-byte frame liblz4 itself emits (content size omitted).
+ * chunk yields the 11-byte frame liblz4 itself emits (content size omitted).  SKY_F_LINKED: FLG=0x48 (linked blocks).
  */
 #ifndef SKYCHUNK_H
 #define SKYCHUNK_H
@@ -63,6 +63,12 @@ extern "C" {
  * e2ee_key_bytes (gateway_operator.py:183-186, :362-364) and the receiver undoes (gateway_receiver.py:191-193). */
 #define SKY_F_E2EE 16u
 #define SKY_BOX_OVERHEAD 40u
+/* linked blocks (sky_submit_flags / sky_process_device): a block's matches may also reach into the 4 KiB of input before
+ * it (sky_kernel_config(4)), as the reference's frames do -- FLG 0x48 instead of 0x68 for chunks of more than one block,
+ * a better ratio on text, and the receiver decodes the blocks of a chunk in order.  A chunk of at most 64 KiB gets the
+ * same FLG as liblz4 gives it (0x68).  Composes with SKY_F_E2EE (the box holds the linked frame); no effect without
+ * SKY_F_LZ4.  sky_frame_bound / sky_box_bound are unchanged. */
+#define SKY_F_LINKED 32u
 
 typedef struct sky_ctx sky_ctx;
 
@@ -76,8 +82,9 @@ SKY_API int sky_device_count(int *count);
  * unlike nvidia-smi -i); the host side maps it to the GPU's NUMA node before pinning staging memory. */
 SKY_API int sky_device_pci_bus_id(int device, char *buf, int len);
 /* Compile-time constants of the kernels in this build (tuning builds differ): what = 0 -> LZ4 match-table entries per
- * CTA, 1 -> warps per CTA of the fused kernel, 2 -> probe slots per segment, 3 -> log2 of the largest probe stride.
- * Unknown `what` returns 0.  Parity tests feed these to the sequential twin of the compressor (tools/lz4_tile_model.c). */
+ * CTA, 1 -> warps per CTA of the fused kernel, 2 -> probe slots per segment, 3 -> log2 of the largest probe stride,
+ * 4 -> SKY_F_LINKED window bytes (0 = no linked mode in this build), 5 -> log2 of the stride at which the window seeds
+ * the match table, 6 -> match-table entries in linked mode.  Unknown `what` returns 0.  Parity tests feed these to the sequential twin of the compressor (tools/lz4_tile_model.c). */
 SKY_API uint32_t sky_kernel_config(int what);
 
 /* Worst-case frame bytes for an n-byte chunk: 15 + n + 4*ceil(n/65536) + 4 (11 when n == 0). */

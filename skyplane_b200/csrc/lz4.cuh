@@ -8,7 +8,8 @@
 //   * the match table is 4096 x (pos16 << 16 | tag16) in shared memory; a probe never reads the candidate's bytes;
 //   * 32 probe slots are one warp instruction; the stride between slots doubles over data without hits;
 //   * parser warps verify and extend the hits of whole segments independently and emit standard LZ4 sequences;
-//   * blocks that do not shrink are stored raw (bit 31 of the block header), like LZ4F_makeBlock.
+//   * blocks that do not shrink are stored raw (bit 31 of the block header), like LZ4F_makeBlock;
+//   * linked blocks (SKY_F_LINKED): the block is parsed behind a window of the input before it (parse_segment).
 // Output is a standard LZ4 block: decodable by lz4.frame.decompress (gateway_receiver.py:196).
 // tools/lz4_tile_model.c is the sequential twin of the parse; frames are byte-identical to it (tests).
 #pragma once
@@ -146,9 +147,10 @@ __device__ __forceinline__ uint32_t xxh32_small(const uint8_t *p, uint32_t len) 
     return h;
 }
 
-// Writes the frame header for an n-byte chunk at dst; returns its size (15, or 7 when n == 0).
-// Single thread.
-__device__ __forceinline__ uint32_t write_frame_header(uint8_t *dst, uint64_t n) {
+// Writes the frame header for an n-byte chunk at dst; returns its size (15, or 7 when n == 0).  linked: FLG 0x48 (linked
+// blocks) when the chunk has more than one block; one block keeps 0x68, as LZ4F_compressFrame switches a single-block
+// input to independent blocks.  Single thread.
+__device__ __forceinline__ uint32_t write_frame_header(uint8_t *dst, uint64_t n, bool linked = false) {
     uint8_t d[10];
     d[1] = 0x40;  // BD: 64 KiB blocks
     dst[0] = 0x04; dst[1] = 0x22; dst[2] = 0x4D; dst[3] = 0x18;
@@ -158,7 +160,7 @@ __device__ __forceinline__ uint32_t write_frame_header(uint8_t *dst, uint64_t n)
         dst[6] = (uint8_t)(xxh32_small(d, 2) >> 8);
         return 7;
     }
-    d[0] = 0x68;  // v01 | B.Indep | C.Size
+    d[0] = linked && n > kBlock ? 0x48 : 0x68;  // v01 | C.Size (| B.Indep)
 #pragma unroll
     for (int i = 0; i < 8; i++) d[2 + i] = (uint8_t)(n >> (8 * i));
 #pragma unroll
@@ -342,6 +344,8 @@ __device__ __forceinline__ uint32_t extend_coop_s(uint32_t in32, uint32_t mpos, 
 // lane writes its own token, length bytes, literals (runs >= kCoopLit: one warp copy each), offset and match-length bytes.
 // skip_first: lane 0 holds the segment's FIRST sequence, which is not emitted here (its literal run is completed with the
 // literals carried over from earlier segments when the block is assembled).
+// (One copy per kernel: kLinked only keeps the linked kernel's call from changing how the default kernel's is compiled.)
+template <bool kLinked>
 __device__ __noinline__ uint32_t flush_seqs(uint8_t *__restrict__ out, uint32_t op, const uint8_t *in, uint32_t q0, uint32_t q1,
                                             uint32_t nseq, bool skip_first, unsigned lane) {
     const uint32_t in32 = smem_u32(in);
@@ -419,6 +423,11 @@ __device__ __noinline__ uint32_t flush_seqs(uint8_t *__restrict__ out, uint32_t 
 // Slots past the last probe position (p > mflimit, only at the very end of a block, always the highest lanes) hash a
 // clamped position: the entries they leave in the table no later lookup can observe, and the hits they report the parser
 // masks out (parse_segment), so the prober spends nothing on them.
+// kLinked (positions are window coordinates, up to window + 64 KiB, kept modulo 65536 in the entry): every lane first
+// stores its entry, then max-es it in.  The store replaces whatever an earlier group left, which the max alone would keep
+// once positions wrap; the max then picks the group's last slot.  A group never straddles the wrap (window coordinate
+// 65536 = block position 65536 - W, a multiple of 1024 and so a group boundary), so the max sees no wrap inside a group.
+// The offset (mine - e) >> 16 is then (position - entry) mod 65536: always 1..65535 for a hit.
 __device__ __forceinline__ uint32_t bfind(uint32_t x) {  // index of the highest set bit (0xffffffff for 0): one FLO
     uint32_t r;
     asm("bfind.u32 %0, %1;" : "=r"(r) : "r"(x));
@@ -446,7 +455,7 @@ __device__ __forceinline__ void near_slot(uint32_t &n, uint32_t hf, uint32_t c3,
 __device__ __forceinline__ void red_max_s(uint32_t a, uint32_t v) {
     asm volatile("red.shared.max.u32 [%0], %1;" ::"r"(a), "r"(v) : "memory");
 }
-template <class Turn>
+template <bool kLinked = false, class Turn>
 __device__ __forceinline__ uint32_t probe_batch(uint32_t in_s, uint32_t tab_s, uint32_t offs_s, uint32_t masks_s, uint32_t seg_pos,
                                                 uint32_t slog, uint32_t batch, uint32_t mflimit, unsigned lane, Turn turn) {
     const uint32_t pstep = 32u << slog;
@@ -474,6 +483,10 @@ __device__ __forceinline__ uint32_t probe_batch(uint32_t in_s, uint32_t tab_s, u
     for (int k = 0; k < 8; k++) {
         e[k] = lds32(tab_s + idx[k]);
         __syncwarp();  // (orders the lanes' table reads of this group before its updates)
+        if (kLinked) {
+            sts32(tab_s + idx[k], mine[k]);
+            __syncwarp();
+        }
         red_max_s(tab_s + idx[k], mine[k]);
         __syncwarp();
     }
@@ -492,8 +505,12 @@ __device__ __forceinline__ uint32_t probe_batch(uint32_t in_s, uint32_t tab_s, u
 
 // ---- parser: one segment.  in = shared-memory copy of the block, scr = this segment's scratch area.
 // (Hits only exist at positions <= L-12 inside the segment, so a hit position is always below the match limit.)
+// Linked blocks: in = [window | block], base = the window's length, L = base + block length; positions are window
+// coordinates, so candidates (and the backward extension's min(pos - anchor, cand, 8)) may reach into the window.  What
+// the segment hands on (record, literal starts) is relative to the block.
+template <bool kLinked = false>
 __device__ __forceinline__ SegRec parse_segment(const uint8_t *in, const SegSlot *slot, uint8_t *__restrict__ scr, uint32_t L,
-                                                unsigned lane) {
+                                                unsigned lane, uint32_t base = 0) {
     const uint32_t in32 = smem_u32(in), offs_s = smem_u32(slot->offs);
     const uint32_t seg_pos = slot->seg_pos, slog = slot->slog;
     const uint32_t mflimit = L - kMfLimit, matchlimit = L - kLastLiterals;
@@ -544,7 +561,7 @@ __device__ __forceinline__ SegRec parse_segment(const uint8_t *in, const SegSlot
         const uint32_t end = pos + mlen;
         pos -= back;
         mlen += back;
-        const uint32_t r0 = (pos - anchor) | (mlen << 16), r1 = anchor | (off << 16);
+        const uint32_t r0 = (pos - anchor) | (mlen << 16), r1 = (anchor - base) | (off << 16);
         if (lane == nseq) {
             q0 = r0;
             q1 = r1;
@@ -556,7 +573,7 @@ __device__ __forceinline__ SegRec parse_segment(const uint8_t *in, const SegSlot
                 first_q0 = __shfl_sync(kFull, q0, 0);
                 first_q1 = __shfl_sync(kFull, q1, 0);
             }
-            mbytes = flush_seqs(scr, mbytes, in, q0, q1, 32, first_pending, lane);
+            mbytes = flush_seqs<kLinked>(scr, mbytes, in + base, q0, q1, 32, first_pending, lane);
             first_pending = false;
             nseq = 0;
         }
@@ -566,10 +583,10 @@ __device__ __forceinline__ SegRec parse_segment(const uint8_t *in, const SegSlot
             first_q0 = __shfl_sync(kFull, q0, 0);
             first_q1 = __shfl_sync(kFull, q1, 0);
         }
-        mbytes = flush_seqs(scr, mbytes, in, q0, q1, nseq, first_pending, lane);
+        mbytes = flush_seqs<kLinked>(scr, mbytes, in + base, q0, q1, nseq, first_pending, lane);
     }
     SegRec r;
-    r.seg_pos = seg_pos;
+    r.seg_pos = seg_pos - base;
     r.lead_ml = first_q0;                                            // lead literals | match length << 16 (0: no match)
     r.off_t = (first_q1 >> 16) | ((seg_end - anchor) << 16);        // offset | trailing literals << 16
     r.mbytes = mbytes;

@@ -55,13 +55,27 @@ constexpr int kThreads = kWarps * 32;
 #ifndef SKY_RING_EXTRA
 #define SKY_RING_EXTRA 2
 #endif
-constexpr int kRing = kParsers + SKY_RING_EXTRA;       // segment slots between the prober and the parsers
 constexpr int kMd5WarpsPerCta = 4;        // digest CTAs run 4 MD5 groups (one per SM sub-partition), see sky_fused_kernel
 constexpr uint32_t kRingBytes = SKY_MD5_SLOTS * 2048;  // MD5 staging ring: slots x 64 B x 32 lanes
 constexpr uint32_t kLoadPiece = 8192;     // bytes per bulk copy of the block load
 constexpr int kCtasPerSm = 2;             // fused kernel: 2 x ~110 KiB of shared memory per SM
 constexpr int kOffBits = 40;
 constexpr uint64_t kOffMask = (1ull << kOffBits) - 1;
+
+// Linked blocks (SKY_F_LINKED): block j >= 1 of a chunk is parsed with the kLinkedWindow raw bytes before it in shared
+// memory ([window | block]), the table seeded with every (1 << kLinkedSeedLog)-th window position.  The window is what
+// fits next to a 4096-entry table once the linked kernel gives up the ring's spare slots (DESIGN.md §4.2: a smaller
+// table loses more ratio than a larger window gains).  A multiple of 1024, so that no probe group straddles the point
+// where window coordinates wrap modulo 65536 (probe_batch).
+#ifndef SKY_LINKED_WINDOW
+#define SKY_LINKED_WINDOW 4096
+#endif
+#ifndef SKY_LINKED_SEED_LOG
+#define SKY_LINKED_SEED_LOG 0
+#endif
+constexpr uint32_t kLinkedWindow = SKY_LINKED_WINDOW;
+constexpr uint32_t kLinkedSeedLog = SKY_LINKED_SEED_LOG;
+static_assert(kLinkedWindow % 1024 == 0 && kLinkedWindow <= kBlock, "SKY_LINKED_WINDOW must be a multiple of 1024, at most 64 KiB");
 
 // ---- shared-memory layout of the fused kernel (dynamic, 128-byte aligned base) -------------------------
 struct BlockDesc {            // written by the prober's lane 0, read by every warp after the block-start barrier
@@ -70,6 +84,7 @@ struct BlockDesc {            // written by the prober's lane 0, read by every w
     uint32_t c, j, L, last;   // chunk, block index, block length, 1 = last block of the chunk
     uint32_t valid, pad;
 };
+template <int kRing>
 struct Ctl {
     uint64_t in_full;               // bulk copy of the block has landed
     uint64_t full[kRing], empty[kRing];
@@ -81,17 +96,25 @@ struct Ctl {
     uint32_t csize, raw, last_lits, tail_off;   // plan results: compressed size, stored?, final literal run and where it goes
     uint32_t data_lo, data_hi;                  // frame offset of the block's first data byte
 };
-constexpr uint32_t kInBytes = kBlock + 128;    // + slack: unaligned 4-byte reads may touch the word after the last byte
-constexpr uint32_t kInOff = 0;
-constexpr uint32_t kTabOff = kInOff + kInBytes;
-constexpr uint32_t kRingOff = kTabOff + kTableBytes;
-constexpr uint32_t kRecOff = kRingOff + kRing * (uint32_t)sizeof(SegSlot);
-constexpr uint32_t kPlanOff = kRecOff + kMaxSegs * (uint32_t)sizeof(SegRec);
-constexpr uint32_t kCtlOff = kPlanOff + kMaxSegs * (uint32_t)sizeof(SegPlan);
-constexpr uint32_t kSmemBytes = (kCtlOff + (uint32_t)sizeof(Ctl) + 127u) & ~127u;
-static_assert(kSmemBytes <= 232448 / 2 - 1024, "two CTAs per SM need <= 112.5 KiB each: lower SKY_PARSERS or SKY_LZ4_ENTRIES");
+// kLinked: the block buffer has room for the window in front of the block, paid for by the ring's spare slots.
+template <bool kLinked>
+struct Smem {
+    static constexpr int kRing = kParsers + (kLinked ? 0 : SKY_RING_EXTRA);  // segment slots between the prober and the parsers
+    static constexpr uint32_t kWin = kLinked ? kLinkedWindow : 0;
+    static constexpr uint32_t kInBytes = kWin + kBlock + 128;  // + slack: unaligned 4-byte reads may touch the word after the last byte
+    static constexpr uint32_t kInOff = 0;
+    static constexpr uint32_t kTabOff = kInOff + kInBytes;
+    static constexpr uint32_t kRingOff = kTabOff + kTableBytes;
+    static constexpr uint32_t kRecOff = kRingOff + kRing * (uint32_t)sizeof(SegSlot);
+    static constexpr uint32_t kPlanOff = kRecOff + kMaxSegs * (uint32_t)sizeof(SegRec);
+    static constexpr uint32_t kCtlOff = kPlanOff + kMaxSegs * (uint32_t)sizeof(SegPlan);
+    static constexpr uint32_t kBytes = (kCtlOff + (uint32_t)sizeof(Ctl<kRing>) + 127u) & ~127u;
+    static_assert(kBytes <= 232448 / 2 - 1024, "two CTAs per SM need <= 112.5 KiB each: lower SKY_PARSERS, SKY_LZ4_ENTRIES or SKY_LINKED_WINDOW");
+    static_assert(kMd5WarpsPerCta * kRingBytes <= kInBytes, "the MD5 rings live in the block buffer of a digest CTA");
+};
+constexpr uint32_t kSmemBytes = Smem<false>::kBytes;
+constexpr uint32_t kLinkedSmemBytes = Smem<true>::kBytes;
 static_assert(kEntries % 128 == 0, "SKY_LZ4_ENTRIES must be a multiple of 128");
-static_assert(kMd5WarpsPerCta * kRingBytes <= kInBytes, "the MD5 rings live in the block buffer of a digest CTA");
 static_assert(sizeof(SegSlot) % 16 == 0 && sizeof(SegRec) == 16 && sizeof(SegPlan) == 16, "layout");
 
 struct ChunkDesc {
@@ -147,6 +170,7 @@ __device__ __forceinline__ uint32_t ld_relaxed32(const uint32_t *p) {
 
 // Prober lane 0: claim the next block that has LZ4 work (empty chunks are finished on the spot), wait until the chunk's
 // MD5 lanes are close (so the block is read from HBM once), and describe it to the CTA.
+template <bool kLinked>
 __device__ __forceinline__ void claim_block(const Params &p, BlockDesc *d, bool pace) {
     const uint32_t total = p.rows * p.n_chunks;
     for (;;) {
@@ -190,7 +214,7 @@ __device__ __forceinline__ void claim_block(const Params &p, BlockDesc *d, bool 
         d->L = (uint32_t)min((uint64_t)kBlock, cd.len - boff);
         d->last = (j + 1 == cd.nblk);
         d->valid = 1;
-        if (j == 0) write_frame_header(cd.dst, cd.len);
+        if (j == 0) write_frame_header(cd.dst, cd.len, kLinked);
         return;
     }
 }
@@ -203,15 +227,21 @@ __device__ __forceinline__ void claim_block(const Params &p, BlockDesc *d, bool 
 // OFF chain (per chunk): (next block index << 40) | frame offset of that block -- a prefix sum handed from block j-1 to
 // block j as soon as j-1 knows its compressed size.  Waiting is deadlock-free: a CTA only waits on lower-numbered work
 // items, all of which were claimed earlier by running CTAs.
-__global__ void __launch_bounds__(kThreads, 2) sky_fused_kernel(const Params p) {
+// kLinked (sky_fused_linked_kernel): block j >= 1 is parsed behind its window (lz4.cuh parse_segment), frames get FLG 0x48.
+// Each block's window is raw input, already in HBM: no block waits on another block's compression.
+template <bool kLinked>
+__device__ __forceinline__ void fused_body(const Params &p) {
+    using S = Smem<kLinked>;
+    constexpr int kRing = S::kRing;
+    constexpr uint32_t kInOff = S::kInOff, kTabOff = S::kTabOff, kRingOff = S::kRingOff;
     extern __shared__ __align__(128) uint8_t smem[];
     const unsigned warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     uint8_t *in = smem + kInOff;
     uint32_t *tab = reinterpret_cast<uint32_t *>(smem + kTabOff);
     SegSlot *ring = reinterpret_cast<SegSlot *>(smem + kRingOff);
-    SegRec *recs = reinterpret_cast<SegRec *>(smem + kRecOff);
-    SegPlan *plans = reinterpret_cast<SegPlan *>(smem + kPlanOff);
-    Ctl *ctl = reinterpret_cast<Ctl *>(smem + kCtlOff);
+    SegRec *recs = reinterpret_cast<SegRec *>(smem + S::kRecOff);
+    SegPlan *plans = reinterpret_cast<SegPlan *>(smem + S::kPlanOff);
+    Ctl<kRing> *ctl = reinterpret_cast<Ctl<kRing> *>(smem + S::kCtlOff);
     uint32_t smem_s = smem_u32(smem);  // shared-window address of the CTA's buffer, kept in a register: left to itself the
     asm volatile("" : "+r"(smem_s));   // compiler re-derives it (S2UR SR_CgaCtaId + ULEA) at the top of every prober batch
 
@@ -261,7 +291,7 @@ __global__ void __launch_bounds__(kThreads, 2) sky_fused_kernel(const Params p) 
     for (uint32_t it = 0;; it++) {
         BlockDesc *dsc = &ctl->desc[it & 1];
         if (warp == 0 && lane == 0) {
-            claim_block(p, dsc, pace);
+            claim_block<kLinked>(p, dsc, pace);
             ctl->block_end_seq = 0xffffffffu;
             ctl->nseg = 0;
         }
@@ -269,6 +299,7 @@ __global__ void __launch_bounds__(kThreads, 2) sky_fused_kernel(const Params p) 
         if (!dsc->valid) break;
         const uint8_t *src = dsc->src;
         const uint32_t L = dsc->L;
+        const uint32_t base = kLinked && dsc->j > 0 ? S::kWin : 0u;  // window bytes in front of the block in shared memory
 
         if (warp < kProbers) {
             // ---------------------------------------------------------------- probers (warps 0 and 1, alternate batches of every segment)
@@ -276,9 +307,10 @@ __global__ void __launch_bounds__(kThreads, 2) sky_fused_kernel(const Params p) 
                 if (lane == 0) {
                     const uint32_t bytes = (L + 15u) & ~15u;  // (the input slab is readable up to the next multiple of 16)
                     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic reads of the old block before the async write
-                    mbar_arrive_expect_tx(&ctl->in_full, bytes);
+                    mbar_arrive_expect_tx(&ctl->in_full, bytes + base);
+                    if (kLinked && base) bulk_load(in, src - base, base, &ctl->in_full);  // the window: the raw bytes before the block
                     for (uint32_t o = 0; o < bytes; o += kLoadPiece)  // several copies in flight: the pieces stream in parallel
-                        bulk_load(in + o, src + o, min(kLoadPiece, bytes - o), &ctl->in_full);
+                        bulk_load(in + base + o, src + o, min(kLoadPiece, bytes - o), &ctl->in_full);
                 }
                 // clear the table meanwhile: entry 0 = (position 0, tag 0) doubles as "empty".  (Warp 1's first table access
                 // follows warp 0's first table phase through the token, so it sees the cleared table.)
@@ -290,10 +322,20 @@ __global__ void __launch_bounds__(kThreads, 2) sky_fused_kernel(const Params p) 
             }
             mbar_wait(&ctl->in_full, in_phase);
             in_phase ^= 1;
+            if constexpr (kLinked) {
+                if (warp == 0 && base && L >= kMfLimit + 1) {
+                    // seed the table with the window: inserts only, no hits (positions < 65536 here: the max keeps the last)
+                    for (uint32_t q = lane << kLinkedSeedLog; q < S::kWin; q += 32u << kLinkedSeedLog) {
+                        const uint32_t hf = load32s(smem_s + kInOff, q) * 2654435761u + lds8(smem_s + kInOff + q + 4) * 0x85EBCA6Bu;
+                        red_max_s(smem_s + kTabOff + __umulhi(hf, kEntries) * 4u, __byte_perm(q, hf, 0x1065));
+                    }
+                    __syncwarp();
+                }
+            }
             uint32_t nseg = 0;
             if (L >= kMfLimit + 1) {
-                const uint32_t mflimit = L - kMfLimit;
-                uint32_t seg_pos = 0, slog = 0;
+                const uint32_t mflimit = base + L - kMfLimit;
+                uint32_t seg_pos = base, slog = 0;
                 while (seg_pos <= mflimit) {
                     if (nseg >= 2) {  // the verdict on segment nseg-2 decides this segment's stride
                         const bool h = ctl->seg_hit[(nseg - 2) & 3u] != 0u;
@@ -304,7 +346,7 @@ __global__ void __launch_bounds__(kThreads, 2) sky_fused_kernel(const Params p) 
 #pragma unroll 1
                     for (uint32_t b = warp; b < 4; b += kProbers) {
                         const uint32_t slot_s = smem_s + kRingOff + si * (uint32_t)sizeof(SegSlot);
-                        const uint32_t hits = probe_batch(smem_s + kInOff, smem_s + kTabOff, slot_s + (uint32_t)offsetof(SegSlot, offs),
+                        const uint32_t hits = probe_batch<kLinked>(smem_s + kInOff, smem_s + kTabOff, slot_s + (uint32_t)offsetof(SegSlot, offs),
                                                           slot_s + (uint32_t)offsetof(SegSlot, masks), seg_pos, slog, b, mflimit, lane, [&]() {
                             // my turn at the table: the other prober has finished the previous batch
                             if (warp == 0) {
@@ -363,8 +405,8 @@ __global__ void __launch_bounds__(kThreads, 2) sky_fused_kernel(const Params p) 
                 if (!got) break;
                 const SegSlot *slot = ring + si;
                 const uint32_t sidx = slot->sidx;
-                uint8_t *scr = scratch + slot->seg_pos + sidx * kSegPad;
-                const SegRec r = parse_segment(in, slot, scr, L, lane);
+                uint8_t *scr = scratch + (slot->seg_pos - base) + sidx * kSegPad;
+                const SegRec r = parse_segment<kLinked>(in, slot, scr, base + L, lane, base);
                 __syncwarp();
                 if (lane == 0) {
                     mbar_arrive(&ctl->empty[si]);
@@ -507,6 +549,9 @@ __global__ void __launch_bounds__(kThreads, 2) sky_fused_kernel(const Params p) 
         }
     }
 }
+
+__global__ void __launch_bounds__(kThreads, 2) sky_fused_kernel(const Params p) { fused_body<false>(p); }
+__global__ void __launch_bounds__(kThreads, 2) sky_fused_linked_kernel(const Params p) { fused_body<true>(p); }
 
 
 // ------------------------------------------------------------------------------------ receiver side
@@ -861,6 +906,9 @@ uint32_t sky_kernel_config(int what) {
     case 1: return (uint32_t)kWarps;
     case 2: return kSegSlots;
     case 3: return kMaxStepLog;
+    case 4: return kLinkedWindow;
+    case 5: return kLinkedSeedLog;
+    case 6: return kEntries;  // the linked kernel keeps the default table
     default: return 0;
     }
 }
@@ -915,6 +963,8 @@ static int init_ctx(sky_ctx *ctx, uint64_t max_batch_bytes, uint32_t n_slots) {
     ctx->sm_count = prop.multiProcessorCount;
     cudaError_t e = cudaFuncSetAttribute(sky_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(sky_fused_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(sky_fused_linked_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLinkedSmemBytes);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(sky_fused_linked_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
     if (e != cudaSuccess) return fail(ctx, SKY_E_CUDA, "cudaFuncSetAttribute(smem) -> %s (built for sm_100a only)", cudaGetErrorString(e));
     // every chunk is placed at a 16-byte aligned offset; frames need bound(len) each
     const uint64_t max_chunks = ctx->max_chunks;
@@ -1080,7 +1130,8 @@ static int launch_batch(sky_ctx *ctx, Slot &s, cudaStream_t st, cudaStream_t met
     p.rows = rows;
     p.flags = flags;
     CK(ctx, cudaEventRecord(s.ev_k0, st));
-    sky_fused_kernel<<<grid, kThreads, kSmemBytes, st>>>(p);
+    if ((flags & SKY_F_LINKED) && (flags & SKY_F_LZ4)) sky_fused_linked_kernel<<<grid, kThreads, kLinkedSmemBytes, st>>>(p);
+    else sky_fused_kernel<<<grid, kThreads, kSmemBytes, st>>>(p);
     CK(ctx, cudaGetLastError());
     CK(ctx, cudaEventRecord(s.ev_k1, st));
     ctx->launches++;

@@ -14,7 +14,7 @@ LIB_PATH = _PKG / "libskychunk.so"
 
 SKY_OK = 0
 SKY_E_INVALID, SKY_E_NOGPU, SKY_E_CUDA, SKY_E_CAPACITY, SKY_E_BUSY, SKY_E_TICKET, SKY_E_NOMEM, SKY_E_NOKEY = -1, -2, -3, -4, -5, -6, -7, -8
-F_LZ4, F_MD5, F_MD5_EXCLUSIVE, F_NO_PACING, F_E2EE = 1, 2, 4, 8, 16
+F_LZ4, F_MD5, F_MD5_EXCLUSIVE, F_NO_PACING, F_E2EE, F_LINKED = 1, 2, 4, 8, 16, 32
 BOX_OVERHEAD = 40
 # sky_decode status codes
 D_OK, D_BAD_HEADER, D_CORRUPT, D_SIZE, D_UNSUPPORTED, D_LAYOUT, D_TRUNCATED, D_AUTH = 0, -1, -2, -3, -4, -5, -6, -7
@@ -106,10 +106,17 @@ def device_pci_bus_id(device: int) -> str:
 
 
 def kernel_config() -> dict:
-    """Compile-time constants of the loaded build (sky_kernel_config)."""
+    """Compile-time constants of the loaded build (sky_kernel_config).  linked_window = 0: no F_LINKED in this build."""
     L = lib()
     return {"lz4_entries": L.sky_kernel_config(0), "warps": L.sky_kernel_config(1), "seg_slots": L.sky_kernel_config(2),
-            "max_step_log": L.sky_kernel_config(3)}
+            "max_step_log": L.sky_kernel_config(3), "linked_window": L.sky_kernel_config(4),
+            "linked_seed_log": L.sky_kernel_config(5), "linked_entries": L.sky_kernel_config(6)}
+
+
+def require_linked() -> None:
+    """Raise unless the loaded build has F_LINKED (a build without it would send independent frames)."""
+    if not kernel_config()["linked_window"]:
+        raise SkyChunkError(SKY_E_INVALID, "this libskychunk build has no linked-block mode (sky_kernel_config(4) == 0)")
 
 
 def frame_bound(n: int) -> int:

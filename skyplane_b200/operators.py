@@ -133,15 +133,19 @@ class GatewayCompressHash(GatewayOperator):
         e2ee_key_bytes: Optional[bytes] = None,
         sink=None,
         n_slots: int = 4,
+        block_linked: bool = False,
     ):
         """use_compression / e2ee_key_bytes: GatewaySender's arguments of the same name (gateway_operator.py:154-168):
         ``use_compression=False`` digests the chunk and lets it pass through uncompressed (``is_compressed=False``);
         ``e2ee_key_bytes`` seals every payload in a SecretBox on the GPU.
         sink: ``callable(worker_id) -> socket``, called once in each worker.  With a sink the worker sends every payload
         straight from the pinned staging slot (``wire.send_results``: WireProtocolHeader + payload, no intermediate bytes
-        object, no frame file) -- the tail of ``GatewaySender.process`` (gateway_operator.py:367-402)."""
+        object, no frame file) -- the tail of ``GatewaySender.process`` (gateway_operator.py:367-402).
+        block_linked: linked-block frames (``native.F_LINKED``), a few percent smaller on text; any LZ4 frame decoder, and
+        so the receiver, reads them unchanged.  Raises when the worker creates its stage on a build without linked mode."""
         super().__init__(handle, region, input_queue, output_queue, error_event, error_queue, chunk_store, n_processes)
         self.use_compression = True if use_compression is None else bool(use_compression)
+        self.block_linked = bool(block_linked)
         self.e2ee_key_bytes = e2ee_key_bytes
         self.sink = sink
         # batches in flight per worker: a batch of 8 MiB chunks spends >= 70 ms on the GPU whatever its size (one serial MD5
@@ -172,6 +176,8 @@ class GatewayCompressHash(GatewayOperator):
                 from skyplane_b200.numa import bind_to_gpu
 
                 bind_to_gpu(device)  # pinned staging buffers on the GPU's own socket
+            if self.block_linked:
+                native.require_linked()
             self._stage = ChunkStage(device, self.max_batch_bytes, self.max_batch_chunks, n_slots=self.n_slots)
             if self.e2ee_key_bytes is not None:
                 self._stage.set_e2ee_key(self.e2ee_key_bytes)
@@ -284,7 +290,8 @@ class GatewayCompressHash(GatewayOperator):
         if not all([fut.result() for _, fut in jobs]):
             stage.release(slot)
             return False
-        stage.launch(slot, compress=self.use_compression, encrypt=self.e2ee_key_bytes is not None)
+        linked = {"linked": True} if self.block_linked else {}  # (only when asked for: stage look-alikes need not know it)
+        stage.launch(slot, compress=self.use_compression, encrypt=self.e2ee_key_bytes is not None, **linked)
         return True
 
     def _launch(self, reqs: List[ChunkRequest]):

@@ -31,6 +31,7 @@ def _compress_hash(op: Dict, kw: Dict) -> GatewayOperator:
         **kw,
         n_processes=op.get("num_gpus", 1),
         use_compression=op.get("compress", True),
+        block_linked=op.get("block_linked", False),
         max_batch_chunks=op.get("max_batch_chunks", 64),
         max_batch_bytes=op.get("max_batch_bytes", 512 << 20),
         n_gpus=op.get("num_gpus"),

@@ -24,6 +24,13 @@
  *             (or a whole segment without a match) are carried into the next sequence.  Standard LZ4 block format.
  *             A block whose compressed size would exceed L-1 is stored raw (return 0), as LZ4F_makeBlock does.
  *
+ * Linked blocks (tile_compress_block_linked): the block is parsed in a buffer [window | block] whose window is the W raw
+ * bytes before the block.  All positions are window coordinates; the table holds them modulo 65536 (pos16), so an offset
+ * is (position - entry) mod 65536, which keeps every offset in 1..65535.  Before the block's first segment the table is
+ * seeded with the window positions 0, s, 2s, ... (s = 1 << seed_step_log), inserted in order without reporting hits.
+ * After that the parse is the one above: candidates may lie in the window, a match that starts there may run on into the
+ * block, backward extension stops at min(pos - anchor, cand, 8).  With W = 0 it is tile_compress_block exactly.
+ *
  * Build: gcc -O2 -shared -fPIC -o tools/bin/liblz4tile.so tools/lz4_tile_model.c
  */
 #include <stdint.h>
@@ -68,17 +75,22 @@ typedef struct { uint64_t probes, hits, accepted, segments; } tile_stats;
 static tile_stats g_stats;
 void tile_model_stats(tile_stats *s, int reset) { *s = g_stats; if (reset) memset(&g_stats, 0, sizeof g_stats); }
 
-/* returns compressed size, or 0 if the block does not shrink (store raw); out capacity >= L + 2048 */
-uint32_t tile_compress_block(const uint8_t *src, uint32_t L, uint8_t *out, const tile_opts *o) {
-    const uint32_t S = (uint32_t)o->seg_slots, limit = L - 1;
-    uint32_t *tab = calloc((size_t)o->entries, 4);  /* pos | tag << 16 ; 0 = (pos 0, tag 0) = "empty" */
+/* The block is src[base .. base + BL); src[0 .. base) is its window.  Positions are window coordinates (base = 0: block
+ * coordinates).  Returns compressed size, or 0 if the block does not shrink (store raw); out capacity >= BL + 2048. */
+static uint32_t compress_block_at(const uint8_t *src, uint32_t base, uint32_t BL, uint8_t *out, const tile_opts *o, int seed_step_log) {
+    const uint32_t S = (uint32_t)o->seg_slots, limit = BL - 1, L = base + BL;
+    uint32_t *tab = calloc((size_t)o->entries, 4);  /* pos16 | tag << 16 ; 0 = (pos 0, tag 0) = "empty" */
     uint16_t *off = malloc(2 * S);
     uint8_t *hit = malloc(S);
-    uint32_t anchor = 0 /* start of the literals not yet emitted */, op = 0, result = 0;
+    uint32_t anchor = base /* start of the literals not yet emitted */, op = 0, result = 0;
     uint32_t ghf[32];
-    if (L >= MFLIMIT + 1) {
+    if (BL >= MFLIMIT + 1) {
         const uint32_t mflimit = L - MFLIMIT, matchlimit = L - LASTLITERALS;
-        uint32_t seg_pos = 0, slog = 0, slog_next = 0;  /* slog of this segment / of the next one */
+        for (uint32_t q = 0; q < base; q += 1u << seed_step_log) {  /* window seeding: inserts only, the last one stays */
+            const uint32_t hf = hash5(src + q);
+            tab[hidx(hf, o)] = (q & 0xffffu) | (htag(hf) << 16);
+        }
+        uint32_t seg_pos = base, slog = 0, slog_next = 0;  /* slog of this segment / of the next one */
         while (seg_pos <= mflimit) {
             g_stats.segments++;
             /* ---- probe, one group of 32 slots at a time */
@@ -90,20 +102,20 @@ uint32_t tile_compress_block(const uint8_t *src, uint32_t L, uint8_t *out, const
                     ghf[i - g] = 0;
                     if (p > mflimit) continue;
                     const uint32_t hf = hash5(src + p);
-                    const uint32_t e = tab[hidx(hf, o)], epos = e & 0xffffu;
+                    const uint32_t e = tab[hidx(hf, o)], eoff = (p - e) & 0xffffu;  /* (p - entry) mod 65536 */
                     ghf[i - g] = hf;
                     g_stats.probes++;
-                    if ((e >> 16) == htag(hf) && epos < p) { hit[i] = 1; off[i] = (uint16_t)(p - epos); }
+                    if ((e >> 16) == htag(hf) && eoff != 0) { hit[i] = 1; off[i] = (uint16_t)eoff; }
                     if (o->group_lag) {  /* an equal hash 3, 4 or 8 slots back in the group is the nearer candidate */
                         for (uint32_t d = 1; d <= i - g; d++)
                             if ((((uint32_t)o->near_mask >> (d - 1)) & 1u) && ghf[i - g - d] == hf) { hit[i] = 1; off[i] = (uint16_t)(d << slog); break; }
-                    } else tab[hidx(hf, o)] = p | (htag(hf) << 16);
+                    } else tab[hidx(hf, o)] = (p & 0xffffu) | (htag(hf) << 16);
                     if (hit[i]) { anyhit = 1; g_stats.hits++; }
                 }
                 if (o->group_lag)  /* the group's slots replace the table entries in slot order (the last one stays) */
                     for (uint32_t i = g; i < g + 32; i++) {
                         const uint32_t p = seg_pos + (i << slog);
-                        if (p <= mflimit) tab[hidx(ghf[i - g], o)] = p | (htag(ghf[i - g]) << 16);
+                        if (p <= mflimit) tab[hidx(ghf[i - g], o)] = (p & 0xffffu) | (htag(ghf[i - g]) << 16);
                     }
             }
             /* ---- parse: depends on nothing outside this segment */
@@ -131,7 +143,7 @@ uint32_t tile_compress_block(const uint8_t *src, uint32_t L, uint8_t *out, const
                 op = emit(out, op, src, anchor, pos - anchor, mlen, pos - cand);
                 anchor = cur = lanchor = pos + mlen;
                 g_stats.accepted++;
-                if (op > L + 1024) goto done;  /* (model only) hopeless and about to overrun the caller's buffer */
+                if (op > BL + 1024) goto done;  /* (model only) hopeless and about to overrun the caller's buffer */
             }
             seg_pos = seg_lim;
             {   /* this segment's verdict decides the stride two segments on */
@@ -141,10 +153,27 @@ uint32_t tile_compress_block(const uint8_t *src, uint32_t L, uint8_t *out, const
             }
         }
     }
-    if (L - anchor + (L - anchor) / 255 + 2 + op <= L + 2040) op = emit(out, op, src, anchor, L - anchor, 0, 0);
-    else op = L;  /* cannot fit anyway */
+    if (L - anchor + (L - anchor) / 255 + 2 + op <= BL + 2040) op = emit(out, op, src, anchor, L - anchor, 0, 0);
+    else op = BL;  /* cannot fit anyway */
     if (op <= limit) result = op;
 done:
     free(tab); free(off); free(hit);
     return result;
+}
+
+/* returns compressed size, or 0 if the block does not shrink (store raw); out capacity >= L + 2048 */
+uint32_t tile_compress_block(const uint8_t *src, uint32_t L, uint8_t *out, const tile_opts *o) {
+    return compress_block_at(src, 0, L, out, o, 0);
+}
+
+/* Linked block: win = the win_len raw bytes just before src (the previous block's tail; win_len 0 for a frame's first block).
+ * Same return value and out capacity as tile_compress_block. */
+uint32_t tile_compress_block_linked(const uint8_t *win, uint32_t win_len, const uint8_t *src, uint32_t L, uint8_t *out,
+                                    const tile_opts *o, int seed_step_log) {
+    uint8_t *buf = malloc((size_t)win_len + L + 1);
+    memcpy(buf, win, win_len);
+    memcpy(buf + win_len, src, L);
+    const uint32_t r = compress_block_at(buf, win_len, L, out, o, seed_step_log);
+    free(buf);
+    return r;
 }

@@ -1,7 +1,11 @@
 #!/usr/bin/env python
 """Compression ratio of the kernel's parse (its sequential CPU twin, tools/lz4_tile_model.c) on data kinds beyond the bench's
 Silesia-like set, next to liblz4's: linked blocks (what the reference emits) and independent blocks (what any block-parallel
-compressor is limited to).  Development tool: CPU only, reads files that happen to be installed in the build container."""
+compressor is limited to).  Development tool: CPU only, reads files that happen to be installed in the build container.
+
+--linked adds the linked-block twin (tile_model.frame_linked: block j sees the W raw bytes before it, the table seeded
+with every (1 << s)-th window position) for W in LINKED_WINDOWS and s in LINKED_SEED_LOGS; its output is
+profiles/linked_ratio_cpu_twin.jsonl."""
 import glob
 import json
 import os
@@ -49,7 +53,12 @@ def kinds():
     }
 
 
+LINKED_WINDOWS = (4096, 8192, 16384, 32768, 65536)  # 4 KiB: what fits the kernel's shared memory next to a 4096-entry table
+LINKED_SEED_LOGS = (0, 1, 2)
+
+
 if __name__ == "__main__":
+    linked = "--linked" in sys.argv
     for name, d in kinds().items():
         if not d:
             continue
@@ -62,4 +71,10 @@ if __name__ == "__main__":
         if indep:
             row["liblz4_independent_blocks_ratio"] = round(raw / indep, 4)
             row["vs_liblz4_independent"] = round(indep / ours, 4)
+        if linked:
+            for w in LINKED_WINDOWS:
+                for sl in LINKED_SEED_LOGS:
+                    fr = tm.frame_linked(d, tm.kernel_opts(), w, sl)
+                    assert ref.lz4f_decompress(fr, raw) == d
+                    row[f"linked_w{w >> 10}k_seed{1 << sl}_ratio"] = round(raw / len(fr), 4)
         print(json.dumps(row), flush=True)

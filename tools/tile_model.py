@@ -1,5 +1,6 @@
 """Python face of tools/lz4_tile_model.c, the sequential CPU twin of the GPU block compressor (development / test tool,
-not product code).  frame(data) assembles the LZ4 frame the GPU stage must emit byte for byte."""
+not product code).  frame(data) assembles the LZ4 frame the GPU stage must emit byte for byte, frame_linked(data, ...) the
+one it emits with SKY_F_LINKED."""
 from __future__ import annotations
 
 import ctypes
@@ -35,6 +36,9 @@ def lib():
         _lib = ctypes.CDLL(str(_SO))
         _lib.tile_compress_block.argtypes = [ctypes.c_char_p, ctypes.c_uint32, ctypes.c_char_p, ctypes.POINTER(Opts)]
         _lib.tile_compress_block.restype = ctypes.c_uint32
+        _lib.tile_compress_block_linked.argtypes = [ctypes.c_char_p, ctypes.c_uint32, ctypes.c_char_p, ctypes.c_uint32, ctypes.c_char_p,
+                                                    ctypes.POINTER(Opts), ctypes.c_int]
+        _lib.tile_compress_block_linked.restype = ctypes.c_uint32
     return _lib
 
 
@@ -68,13 +72,36 @@ def blocks(data: bytes, o: Opts):
     return out
 
 
-def frame(data: bytes, o: Opts | None = None) -> bytes:
-    o = o or kernel_opts()
+def blocks_linked(data: bytes, o: Opts, W: int, seed_step_log: int):
+    """blocks() for a linked frame: block j >= 1 sees the W raw bytes before it as its window."""
+    L = lib()
+    buf = ctypes.create_string_buffer(65536 + 4096)
+    out = []
+    for pos in range(0, len(data), 65536):
+        blk, win = data[pos:pos + 65536], data[max(0, pos - W):pos]
+        c = L.tile_compress_block_linked(win, len(win), blk, len(blk), buf, ctypes.byref(o), seed_step_log)
+        out.append((c, buf.raw[:c] if c else blk))
+    return out
+
+
+def _frame(data: bytes, flg: int, blks) -> bytes:
     if not data:
         d = bytes([0x60, 0x40])
         return bytes([0x04, 0x22, 0x4D, 0x18]) + d + bytes([(_xxh32_small(d) >> 8) & 0xFF]) + bytes(4)
-    d = bytes([0x68, 0x40]) + len(data).to_bytes(8, "little")
+    d = bytes([flg, 0x40]) + len(data).to_bytes(8, "little")
     fr = bytearray(bytes([0x04, 0x22, 0x4D, 0x18]) + d + bytes([(_xxh32_small(d) >> 8) & 0xFF]))
-    for c, b in blocks(data, o):
+    for c, b in blks:
         fr += (c if c else (len(b) | 0x80000000)).to_bytes(4, "little") + b
     return bytes(fr + bytes(4))
+
+
+def frame(data: bytes, o: Opts | None = None) -> bytes:
+    o = o or kernel_opts()
+    return _frame(data, 0x68, blocks(data, o))
+
+
+def frame_linked(data: bytes, o: Opts | None = None, W: int = 4096, seed_step_log: int = 0) -> bytes:
+    """The frame SKY_F_LINKED emits: FLG 0x48 (linked blocks, content size) when the chunk has more than one block; a chunk
+    of one block gets FLG 0x68 as liblz4 gives it (a single block is independent either way)."""
+    o = o or kernel_opts()
+    return _frame(data, 0x48 if len(data) > 65536 else 0x68, blocks_linked(data, o, W, seed_step_log))
